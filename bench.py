@@ -4,6 +4,8 @@
     python bench.py [--gpus N --steps K --warmup W]            # our arm (CUDA path through the C-ABI)
     python bench.py --impl reference [...]                       # reference arm: the CPU tracker on the host cores
     python bench.py --config {pair_sweep,720p_single,1080p_stress} [--lc-mode const_weight]   # the other BASELINE configs
+    python bench.py [...] --dump-outputs DIR                    # also write the last timed step's result records as DIR/<field>.npy
+                                                                 # (our arm only: the reference arm times a sample of the pairs)
 
 A "step" is one batch of the hot path on one GPU: `frames` new frames (pyramid + gradient texels), `keyframes`
 keyframes (pyramid + mask/count/selection) and `pairs` frame-keyframe tracks (each frame against its own keyframe and
@@ -311,6 +313,27 @@ def run_reference(args, rank, world, conf):
     emit(line)
 
 
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, rec):
+    """The result records a caller of the timed path receives, one DIR/<field>.npy per field of ellc_result (float32; the integer
+    fields as float64, which holds them exactly), so that two builds can be compared output for output.  The workload is seeded,
+    so the same arguments give the same records.  Above DUMP_MAX_BYTES a fixed, seeded sample of the records is written;
+    pair_index.npy holds their positions in the result table."""
+    fields = [n for n in rec.dtype.names if n != "reserved"]
+    row_bytes = 8 + sum(rec.dtype[n].itemsize * (2 if rec.dtype[n].base.kind == "i" else 1) for n in fields)
+    cap = (DUMP_MAX_BYTES - 4096 * (len(fields) + 1)) // row_bytes          # 4 KB per file covers the .npy header
+    idx = np.arange(len(rec))
+    if len(idx) > cap:
+        idx = np.sort(np.random.default_rng(0).choice(len(idx), cap, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pair_index.npy"), idx.astype(np.float64))
+    for n in fields:
+        a = rec[n][idx]
+        np.save(os.path.join(out_dir, n + ".npy"), a.astype(np.float64 if a.dtype.kind == "i" else np.float32))
+
+
 def sass_inst_per_pixel():
     """Static instruction count of the level-0 pixel loop (usual path) from profiles/r02_sass_histogram.json (tools/sass_histogram.py)."""
     try:
@@ -342,7 +365,15 @@ def main():
     ap.add_argument("--exchange-root", type=int, default=0, help="rank that receives all records; -1 = every rank (all-gather)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result records of the last one as DIR/<field>.npy (at most 64 MB); N>1: "
+                         "the table gathered on the --exchange-root rank (rank 0 for -1).  Not with --impl reference, which tracks only "
+                         "a sample of the pair list")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the records of the CUDA path (--impl ours)")
     conf = CONFIGS[args.config]
     W, H = conf["size"]
     if args.config != "pair_sweep":
@@ -805,6 +836,8 @@ def main():
                                 "e2e_ms_per_step": per_rank_ms[1] if len(per_rank_ms) > 1 else None,
                                 "note": "every rank tracks its own seeded segment: iteration counts, hence kernel times, differ a little between ranks"}
         emit(line)
+    if args.dump_outputs and rank == max(root, 0):
+        dump_outputs(args.dump_outputs, table)     # the rank that receives the gathered table (--exchange-root; N = 1: its own records)
     trk.close()
     if world > 1:
         dist.barrier()

@@ -19,12 +19,12 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 
-def reference_case(n_frames=3, seed=31):
-    """Keyframe + frames at the reference's compiled-in size and intrinsics; the last frame is a large rotation (out-of-bounds
-    warps, more iterations)."""
+def reference_case(n_frames=3, seed=31, k=None):
+    """Keyframe + frames at the reference's compiled-in size and intrinsics (`k`: refbinding.dims(), asked of the library when not
+    given); the last frame is a large rotation (out-of-bounds warps, more iterations)."""
     from egomotion_with_local_loop_closures_b200 import synth
     from oracle import refbinding as ref
-    k = ref.dims()
+    k = k or ref.dims()
     kk = dict(fx=k["fx"], fy=k["fy"], cx=k["cx"], cy=k["cy"])
     scene = synth.SynthScene(k["width"], k["height"], k=kk)
     kf = scene.keyframe(noise_seed=seed)

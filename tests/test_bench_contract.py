@@ -1,10 +1,14 @@
-"""CPU: the parts of bench.py's output contract that can be checked without a GPU -- the reference arm (`--impl reference`) runs the
-CPU oracle on a bounded sample of the workload and must print the keys the driver reads, with a `config` that names the WORKLOAD
-only (the same dict our arm prints for the same flags: bench.workload_config)."""
+"""bench.py's output contract.  CPU: the reference arm (`--impl reference`) runs the CPU oracle on a bounded sample of the workload
+and must print the keys of the result line, with a `config` that names the WORKLOAD only (the same dict our arm prints for the same
+flags: bench.workload_config); the --dump-outputs writer.  GPU: --steps sets the number of timed steps, and --dump-outputs writes
+the same records for the same arguments."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -33,3 +37,47 @@ def test_reference_arm_line():
     assert want == line["config"]
     # inputs of the default workload: 512 frames + 32 keyframes (image, 4-level depth and variance) + 4608 pair records
     assert bench.input_bytes_per_step(512, 32, 4608) == 271730688
+
+
+def test_dump_outputs_writer(tmp_path):
+    """One float32 / float64 .npy per field of the result record; a table above 64 MB is written as a fixed, seeded sample."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from egomotion_with_local_loop_closures_b200 import capi
+    rec = np.zeros(400000, capi.RESULT_DTYPE)
+    rec["status"] = np.arange(len(rec))
+    rec["pose"] = np.random.default_rng(1).standard_normal((len(rec), 6))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), rec)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted([n + ".npy" for n in capi.RESULT_DTYPE.names if n != "reserved"] + ["pair_index.npy"])
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 * 10**6
+    idx = np.load(tmp_path / "a" / "pair_index.npy")
+    assert 100000 < len(idx) < len(rec) and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "status.npy"), idx)
+    assert np.array_equal(np.load(tmp_path / "a" / "pose.npy"), rec["pose"][idx.astype(np.int64)])
+    for n in names:
+        a = np.load(tmp_path / "a" / n)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, np.load(tmp_path / "b" / n)), n
+
+
+@pytest.mark.gpu
+def test_steps_and_dump_outputs(tmp_path):
+    """Two runs of the pipelined path that differ only in --steps: the timed region's launches scale with the step count, and the
+    records of the last timed step are identical (seeded inputs, run-to-run deterministic kernels)."""
+    lines = []
+    for steps in (2, 3):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--frames", "32", "--keyframes", "9", "--steps", str(steps),
+                              "--warmup", "1", "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / str(steps))],
+                             capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines.append(json.loads(out.stdout.strip().splitlines()[-1]))
+    assert [l["steps"] for l in lines] == [2, 3] and lines[0]["config"]["pairs_per_gpu_per_step"] == 288
+    assert "alternate" in lines[0]["implementation"]["pipelining"]
+    assert lines[0]["gpu_launches"] > 0 and lines[1]["gpu_launches"] * 2 == lines[0]["gpu_launches"] * 3
+    names = sorted(os.listdir(tmp_path / "2"))
+    assert names == sorted(os.listdir(tmp_path / "3")) and "pose.npy" in names
+    for n in names:
+        a, b = np.load(tmp_path / "2" / n), np.load(tmp_path / "3" / n)
+        assert a.dtype in (np.float32, np.float64) and len(a) == 288 and np.array_equal(a, b), n
+    assert np.all(np.load(tmp_path / "2" / "n_iters.npy").sum(axis=1) > 0) and np.abs(np.load(tmp_path / "2" / "pose.npy")).max() > 0

@@ -6,9 +6,13 @@ oracle/shim/ (oracle/ref_driver.cpp, `make -C oracle ref`).  tests/golden/refere
 produced on seeded inputs at the reference's compiled-in configuration (generator: tests/golden/make_reference_golden.py).
 
   * fixture tests run everywhere (the fixture is committed);
-  * live tests run where the library exists or can be built (this container: /root/reference is mounted).
+  * the tests that take `R` call the reference through it: where the library exists or can be built, R is the library and every
+    call is also checked against tests/golden/reference_live_calls.npz; elsewhere R returns what that file recorded for the
+    call (generator: tests/golden/make_reference_live_golden.py), so the oracle is compared with the reference's outputs
+    everywhere.
 """
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -16,7 +20,15 @@ import pytest
 from oracle import refbinding as ref
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-live = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libellc_ref.so not built and /root/reference not mounted")
+sys.path.insert(0, GOLD)
+from make_reference_live_golden import Replay, same  # noqa: E402
+
+
+@pytest.fixture
+def R(request):
+    """The reference's binding for this test: live where the library is available, its recorded results elsewhere."""
+    variant = "640x480" if "640x480" in request.node.name else "default"
+    return Replay(request.node.name, live=ref if ref.available(variant) else None)
 
 
 @pytest.fixture(scope="module")
@@ -178,23 +190,21 @@ def test_oracle_pyramid_cpp_variant_is_bit_identical_to_the_reference(oracle_mod
         assert np.array_equal(pose_after, g["pyr_poses_after"][c][0]), c
 
 
-# ---- live: the library itself (this container) ----------------------------------------------------------------------------
-@live
-def test_fixture_is_what_the_reference_produces(fx):
+# ---- the library itself, or what it returned (R) ---------------------------------------------------------------------------
+def test_fixture_is_what_the_reference_produces(fx, R):
     g = fx
     depth, var = _depth(g)
-    k = ref.dims()
+    k = R.dims()
     assert (k["width"], k["height"]) == (int(g["width"][0]), int(g["height"][0]))
     assert np.array_equal(np.array([k["fx"], k["fy"], k["cx"], k["cy"]], np.float32), g["intr"])
-    tr = ref.track_trace(g["kf_image"], g["frames"][1], depth, var, g["init"][1], want_weights=True)
+    tr = R.track_trace(g["kf_image"], g["frames"][1], depth, var, g["init"][1], want_weights=True)
     assert tr["n_iters"] == list(g["p1_n_iters"]) and np.array_equal(tr["final_pose"], g["p1_pose"])
-    assert np.array_equal(tr["weights_l0"], g["p1_weights_l0"])
-    pose, po, pw = ref.get_image_pose_estimate(g["kf_image"], g["frames"][1], depth, var, g["init"][1])
+    assert same(tr["weights_l0"], g["p1_weights_l0"])
+    pose, po, pw = R.get_image_pose_estimate(g["kf_image"], g["frames"][1], depth, var, g["init"][1])
     assert np.array_equal(pose, g["p1_driver_pose"]) and np.array_equal(po, g["p1_driver_pose_wrt_origin"])
 
 
-@live
-def test_reference_stages_vs_oracle(oracle_mod, fx):
+def test_reference_stages_vs_oracle(oracle_mod, fx, R):
     """constructImagePyramids / calculateGradient / calculateNonZeroDepthPts (src/Frame.cpp:170-327) on every level, incl. NaN,
     negative and -0 depths."""
     g = fx
@@ -205,17 +215,16 @@ def test_reference_stages_vs_oracle(oracle_mod, fx):
         d = depth[l].copy()
         idx = rng.integers(0, d.size, 40)
         d.reshape(-1)[idx[:10]] = np.nan; d.reshape(-1)[idx[10:20]] = -1.0; d.reshape(-1)[idx[20:30]] = -0.0; d.reshape(-1)[idx[30:]] = np.inf
-        r = ref.frame_level(g["frames"][0], l, d)
-        assert np.array_equal(r["image"], opyr[l]), l
+        r = R.frame_level(g["frames"][0], l, d)
+        assert same(r["image"], opyr[l]), l
         rows, cols = d.shape
         ogx, ogy = oracle_mod.gradient(opyr[l], rows, cols)
-        assert np.array_equal(r["gradx"], ogx) and np.array_equal(r["grady"], ogy), l
+        assert same(r["gradx"], ogx) and same(r["grady"], ogy), l
         omask, ocount = oracle_mod.mask_count(d)
-        assert np.array_equal(r["mask"], omask) and r["count"] == ocount, l
+        assert same(r["mask"], omask) and r["count"] == ocount, l
 
 
-@live
-def test_reference_samplers_vs_oracle(oracle_mod, fx):
+def test_reference_samplers_vs_oracle(oracle_mod, fx, R):
     """frame::getInterpolatedElement (src/Frame.h:181-394) at random, integer, border and out-of-bounds coordinates."""
     g = fx
     img = g["frames"][0]
@@ -226,7 +235,7 @@ def test_reference_samplers_vs_oracle(oracle_mod, fx):
                              [0, cols - 1, cols - 1 + 1e-4, cols - 0.5, -1e-6, -0.5, cols, 0.5]]).astype(np.float32)
         ys = np.concatenate([rng.uniform(-3, rows + 3, 400), rng.integers(-2, rows + 2, 100).astype(np.float64),
                              [0, rows - 1, rows - 1 + 1e-4, rows - 0.5, -1e-6, 2.0, 3.0, rows]]).astype(np.float32)
-        ri, rgx, rgy = ref.interpolate(img, l, xs, ys)
+        ri, rgx, rgy = R.interpolate(img, l, xs, ys)
         lvl = oracle_mod.image_pyramid(img)[l]
         ogx, ogy = oracle_mod.gradient(lvl, rows, cols)
         oi = np.array([oracle_mod.interp_u8(lvl, x, y, 1, rows, cols) for x, y in zip(xs, ys)], np.float32)
@@ -236,25 +245,23 @@ def test_reference_samplers_vs_oracle(oracle_mod, fx):
         assert (ri == -1).sum() > 5 and (ri > 0).sum() > 200
 
 
-@live
-def test_reference_pose_algebra_vs_oracle(oracle_mod):
+def test_reference_pose_algebra_vs_oracle(oracle_mod, R):
     """frame::concatenateRelativePose / concatenateOriginPose (src/Frame.cpp:503-562)."""
     rng = np.random.default_rng(4)
     for n in range(60):
         s = 10.0 ** rng.uniform(-3, 0.3)
         a = (rng.standard_normal(6) * s).astype(np.float32); b = (rng.standard_normal(6) * s).astype(np.float32)
-        assert np.array_equal(ref.concat_relative(a, b), oracle_mod.concat_relative(a, b)), n
-        assert np.array_equal(ref.concat_origin(a, b), oracle_mod.concat_origin(a, b)), n
+        assert np.array_equal(R.concat_relative(a, b), oracle_mod.concat_relative(a, b)), n
+        assert np.array_equal(R.concat_origin(a, b), oracle_mod.concat_origin(a, b)), n
 
 
-@live
-def test_reference_live_random_pairs(oracle_mod):
+def test_reference_live_random_pairs(oracle_mod, R):
     """Fresh seeds (not the fixture's): the oracle stays bit-identical to the reference, including an all-out-of-bounds start
     (zero step: H = 0, cv::Mat::inv() returns zeros) and a keyframe without depth."""
     import sys
     sys.path.insert(0, os.path.join(GOLD))
     from make_reference_golden import reference_case
-    case = reference_case(n_frames=2, seed=77)
+    case = reference_case(n_frames=2, seed=77, k=R.dims())
     k, kf = case["k"], case["kf"]
     ocfg = oracle_mod.default_config(k["width"], k["height"], fx=float(k["fx"]), fy=float(k["fy"]), cx=float(k["cx"]), cy=float(k["cy"]))
     far = np.array([0, 0, 0, 50.0, 0, 0], np.float32)                                        # every warp lands outside the image
@@ -263,7 +270,7 @@ def test_reference_live_random_pairs(oracle_mod):
             (case["frames"][0], kf["depth"], far), (case["frames"][0], nodepth, np.zeros(6, np.float32))]
     for n, (fr, depth, init) in enumerate(runs):
         pose, tr = oracle_mod.track(ocfg, kf["image"], fr, depth, kf["var"], init)
-        r = ref.track_trace(kf["image"], fr, depth, kf["var"], init)
+        r = R.track_trace(kf["image"], fr, depth, kf["var"], init)
         assert tr["n_selected"] == r["n_selected"] and tr["n_iters"] == r["n_iters"], n
         assert np.array_equal(pose, r["final_pose"]), n
         for l in range(4):
@@ -273,19 +280,18 @@ def test_reference_live_random_pairs(oracle_mod):
     assert tr["n_iters"] == [1, 1, 1, 1]                          # no depth: one zero step per level
 
 
-@live
 @pytest.mark.parametrize("parallel", [True, False])
-def test_reference_live_loop_closure_flow(oracle_mod, fx, parallel):
+def test_reference_live_loop_closure_flow(oracle_mod, fx, parallel, R):
     """Both settings of FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST (3 + 2 row bands on threads / one band), a keyframe with three
     saved weight images (1/3 is not a power of two: cv::Mat / scalar multiplies by the float reciprocal)."""
     g = fx
     depth, var = _depth(g)
     ocfg = _ocfg(oracle_mod, g, lc_parallel=int(parallel))
-    r = ref.lc_flow(g["kf_image"], list(g["frames"]), g["init"], depth, var, g["frames"][1], g["gt"][1] * 0.4, parallel=parallel)
+    r = R.lc_flow(g["kf_image"], list(g["frames"]), g["init"], depth, var, g["frames"][1], g["gt"][1] * 0.4, parallel=parallel)
     wf, cnt, seq_poses = _oracle_lc_weights(oracle_mod, g, ocfg)
     assert cnt == r["counts"] and np.array_equal(seq_poses, r["seq_poses"])
     for l in range(4):
-        assert np.array_equal(wf[l], r["weights"][l]), l
+        assert same(r["weights"][l], wf[l]), l
     init = oracle_mod.concat_origin((g["gt"][1] * 0.4).astype(np.float32), np.zeros(6, np.float32))
     pose, tr = oracle_mod.track_lc(ocfg, g["kf_image"], g["frames"][1], depth, wf, init)
     assert np.array_equal(pose, r["lc_pose"]) and np.array_equal(pose, r["lc_trace"]["final_pose"])
@@ -295,14 +301,13 @@ def test_reference_live_loop_closure_flow(oracle_mod, fx, parallel):
             assert np.array_equal(np.asarray(o["H"], np.float32).reshape(6, 6), q["H"]) and np.array_equal(o["b"], q["b"]), l
 
 
-@live
-def test_reference_live_randomised_sweep(oracle_mod):
+def test_reference_live_randomised_sweep(oracle_mod, R):
     """Eight more seeded pairs with random ground-truth motions (0.3 - 4 degrees, up to 0.06 units) and random initial poses,
     forward tracker: counts, iteration counts, every hessian / sd_param / weightedPose / pose bit-identical to the reference."""
     import sys
     sys.path.insert(0, GOLD)
     from egomotion_with_local_loop_closures_b200 import synth
-    k = ref.dims()
+    k = R.dims()
     kk = dict(fx=k["fx"], fy=k["fy"], cx=k["cx"], cy=k["cy"])
     ocfg = oracle_mod.default_config(k["width"], k["height"], fx=float(k["fx"]), fy=float(k["fy"]), cx=float(k["cx"]), cy=float(k["cy"]))
     rng = np.random.default_rng(2026)
@@ -315,7 +320,7 @@ def test_reference_live_randomised_sweep(oracle_mod):
             cur = scene.render(synth.se3_exp(gt), noise_seed=int(rng.integers(1, 10**6)))
             init = (gt * rng.uniform(0.0, 1.2) + rng.normal(0, 1e-3, 6)).astype(np.float32)
             pose, tr = oracle_mod.track(ocfg, kf["image"], cur, kf["depth"], kf["var"], init)
-            r = ref.track_trace(kf["image"], cur, kf["depth"], kf["var"], init)
+            r = R.track_trace(kf["image"], cur, kf["depth"], kf["var"], init)
             assert tr["n_selected"] == r["n_selected"] and tr["n_iters"] == r["n_iters"]
             assert np.array_equal(pose, r["final_pose"])
             for l in range(4):
@@ -327,9 +332,6 @@ def test_reference_live_randomised_sweep(oracle_mod):
 
 
 # ---- the reference's own code at the METRIC resolution (640x480) ----------------------------------------------------------
-live640 = pytest.mark.skipif(not ref.available("640x480"), reason="oracle/_ref/libellc_ref_640x480.so not built and /root/reference not mounted")
-
-
 @pytest.fixture(scope="module")
 def fx640():
     return np.load(os.path.join(GOLD, "reference_track_640x480.npz"))
@@ -373,25 +375,23 @@ def test_oracle_is_bit_identical_to_the_reference_at_640x480(oracle_mod, fx640):
     assert n_it > 20
 
 
-@live640
-def test_fixture_640x480_is_what_the_reference_produces(fx640):
-    prev = ref.select("640x480")
+def test_fixture_640x480_is_what_the_reference_produces(fx640, R):
+    prev = R.select("640x480")
     try:
-        k = ref.dims()
+        k = R.dims()
         assert (k["width"], k["height"], float(k["fx"]), float(k["cx"]), float(k["cy"])) == (640, 480, 512.0, 320.0, 240.0)
         g = fx640
         depth, var = _pyramids640(g)
-        tr = ref.track_trace(g["kf_image"], g["frames"][1], depth, var, g["init"][1])
+        tr = R.track_trace(g["kf_image"], g["frames"][1], depth, var, g["init"][1])
         assert tr["n_iters"] == list(g["p1_n_iters"]) and np.array_equal(tr["final_pose"], g["p1_pose"])
     finally:
-        ref.select(prev)
+        R.select(prev)
 
 
-@live640
-def test_reference_live_random_pairs_at_640x480(oracle_mod, scene_vga):
+def test_reference_live_random_pairs_at_640x480(oracle_mod, scene_vga, R):
     """Fresh pairs at 640x480 (the parity tests' own scene_vga case and two perturbed starts): oracle vs the reference's own code,
     bit-identical at every iteration."""
-    prev = ref.select("640x480")
+    prev = R.select("640x480")
     try:
         case = scene_vga
         ocfg = oracle_mod.default_config(640, 480, fx=512.0, fy=512.0, cx=320.0, cy=240.0)
@@ -401,7 +401,7 @@ def test_reference_live_random_pairs_at_640x480(oracle_mod, scene_vga):
         total = 0
         for n, (fr, init) in enumerate(runs):
             pose, tr = oracle_mod.track(ocfg, kf["image"], fr, kf["depth"], kf["var"], init)
-            r = ref.track_trace(kf["image"], fr, kf["depth"], kf["var"], init)
+            r = R.track_trace(kf["image"], fr, kf["depth"], kf["var"], init)
             assert tr["n_selected"] == r["n_selected"] and tr["n_iters"] == r["n_iters"], n
             assert np.array_equal(pose, r["final_pose"]), n
             for l in range(4):
@@ -411,4 +411,4 @@ def test_reference_live_random_pairs_at_640x480(oracle_mod, scene_vga):
                     total += 1
         assert total > 30
     finally:
-        ref.select(prev)
+        R.select(prev)
