@@ -49,6 +49,13 @@ class IterTrace(C.Structure):
                 ("pad", C.c_int32 * 3)]
 
 
+class Camera(C.Structure):
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("channels", C.c_int32), ("pitch", C.c_int32),
+                ("undistort", C.c_int32), ("reserved", C.c_int32), ("K", C.c_double * 9), ("dist", C.c_double * 5),
+                ("new_K", C.c_double * 9)]
+
+
+assert C.sizeof(Camera) == 208
 assert C.sizeof(Result) == 256 and C.sizeof(IterTrace) == 256 and C.sizeof(Pair) == 36
 
 PAIR_DTYPE = np.dtype([("kf_slot", "<i4"), ("frame_slot", "<i4"), ("init_pose", "<f4", 6), ("flags", "<i4")])
@@ -79,7 +86,8 @@ SYMBOLS = ["ellc_default_config", "ellc_create", "ellc_destroy", "ellc_last_erro
            "ellc_prepare_async", "ellc_batch_kernel_ms", "ellc_batch_interval_ms", "ellc_fence",
            "ellc_exchange_create", "ellc_exchange_attach_ipc", "ellc_exchange_attach_local", "ellc_track_batch_exchange",
            "ellc_exchange_wait", "ellc_exchange_destroy", "ellc_se3_exp_closed", "ellc_se3_log_closed",
-           "ellc_gn_iterate", "ellc_hessian_inverse", "ellc_lc_generate_pairs", "ellc_track_generated_pairs"]
+           "ellc_gn_iterate", "ellc_hessian_inverse", "ellc_lc_generate_pairs", "ellc_track_generated_pairs",
+           "ellc_optimal_new_camera_matrix", "ellc_set_camera", "ellc_ingest_frames", "ellc_ingest_keyframe", "ellc_read_camera_tables"]
 VARIANT_FORWARD, VARIANT_CONST_WEIGHT, VARIANT_PYRAMID = 0, 1, 2
 
 
@@ -168,6 +176,11 @@ def lib():
                                              C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p]
         L.ellc_track_generated_pairs.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
         L.ellc_se3_log_closed.restype = C.c_int
+        L.ellc_optimal_new_camera_matrix.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_double, C.c_void_p]
+        L.ellc_set_camera.argtypes = [C.c_void_p, C.POINTER(Camera)]
+        L.ellc_ingest_frames.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32]
+        L.ellc_ingest_keyframe.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+        L.ellc_read_camera_tables.argtypes = [C.c_void_p] + [C.c_void_p] * 4
         L.ellc_se3_log_closed.argtypes = [C.c_void_p] * 2
         _lib = L
     return _lib
@@ -188,6 +201,30 @@ def default_config(width, height, **over):
         else:
             setattr(cfg, k, v)
     return cfg
+
+
+def optimal_new_camera_matrix(K, dist, width, height, alpha):
+    """cv::getOptimalNewCameraMatrix(K, dist, (width, height), alpha) of OpenCV 3.0.0 (host code)."""
+    K = np.ascontiguousarray(np.asarray(K, np.float64).reshape(9)); d = np.ascontiguousarray(np.asarray(dist, np.float64).reshape(5))
+    out = np.empty(9, np.float64)
+    rc = lib().ellc_optimal_new_camera_matrix(_p(K), _p(d), int(width), int(height), float(alpha), _p(out))
+    if rc != 0:
+        raise EllcError(f"ellc_optimal_new_camera_matrix failed ({rc})")
+    return out.reshape(3, 3)
+
+
+def make_camera(width, height, channels=3, undistort=False, K=None, dist=None, new_K=None, pitch=None):
+    """An ellc_camera record; K / dist / new_K only matter with undistort."""
+    cam = Camera()
+    cam.width, cam.height, cam.channels = int(width), int(height), int(channels)
+    cam.pitch = int(pitch) if pitch is not None else int(width) * int(channels)
+    cam.undistort = 1 if undistort else 0
+    for name, v, n in (("K", K, 9), ("dist", dist, 5), ("new_K", new_K, 9)):
+        if v is not None:
+            arr = getattr(cam, name)
+            for i, x in enumerate(np.asarray(v, np.float64).reshape(n)):
+                arr[i] = float(x)
+    return cam
 
 
 def concat_relative(a, b):
@@ -269,6 +306,61 @@ class Tracker:
         self._keep = getattr(self, "_keep", [])
         self._keep += [image] + d + v
         self._chk(lib().ellc_upload_keyframe(self._h, slot, _p(image), dp, vp))
+
+    # -- camera images (gray + undistortion + resize on the device)
+    def set_camera(self, cam):
+        self._cam = cam
+        self._chk(lib().ellc_set_camera(self._h, C.byref(cam)))
+
+    def _camera_image(self, img):
+        """(pointer, on_device, object to keep alive) of one camera image: a numpy array (host) or a CUDA torch tensor (device),
+        (height, width, channels) or (height, width) uint8, rows contiguous (the camera's pitch = width * channels)."""
+        cam = self._cam
+        shape = (cam.height, cam.width) if cam.channels == 1 else (cam.height, cam.width, cam.channels)
+        if cam.pitch != cam.width * cam.channels:
+            raise EllcError("the Python binding takes unpadded images (pitch = width * channels); the C-ABI takes any pitch")
+        if type(img).__module__.startswith("torch"):
+            import torch
+            if not img.is_cuda or img.dtype != torch.uint8 or not img.is_contiguous() or tuple(img.shape) != shape:
+                raise EllcError(f"camera tensor must be a contiguous uint8 CUDA tensor of shape {shape}")
+            return img.data_ptr(), 1, img
+        a = np.ascontiguousarray(img, np.uint8)
+        if a.shape != shape:
+            raise EllcError(f"camera image shape {a.shape} != {shape}")
+        return a.ctypes.data, 0, a
+
+    def ingest_frames(self, slots, images):
+        """Camera images (all numpy, or all CUDA torch tensors) -> level-0 images of these frame slots."""
+        s = np.ascontiguousarray(slots, np.int32)
+        got = [self._camera_image(im) for im in images]
+        if len({g[1] for g in got}) > 1:
+            raise EllcError("mixed host and device camera images in one call")
+        if got and got[0][1] == 1:
+            import torch
+            torch.cuda.current_stream().synchronize()           # the images must be complete: the library reads them on its own streams
+        ptrs = (C.c_void_p * max(1, len(got)))(*[g[0] for g in got])
+        self._keep = getattr(self, "_keep", []) + [g[2] for g in got]
+        self._chk(lib().ellc_ingest_frames(self._h, len(s), _p(s), ptrs, got[0][1] if got else 0))
+
+    def ingest_keyframe(self, slot, image, depth, var):
+        ptr, dev, keep = self._camera_image(image)
+        if dev:
+            import torch
+            torch.cuda.current_stream().synchronize()
+        d = [np.ascontiguousarray(a, np.float32) for a in depth]
+        v = [np.ascontiguousarray(a, np.float32) for a in var]
+        dp = (C.c_void_p * LEVELS)(*[_p(a) for a in d])
+        vp = (C.c_void_p * LEVELS)(*[_p(a) for a in v])
+        self._keep = getattr(self, "_keep", []) + [keep] + d + v
+        self._chk(lib().ellc_ingest_keyframe(self._h, int(slot), C.c_void_p(ptr), dev, dp, vp))
+
+    def read_camera_tables(self):
+        """(tap_x [width, 2], tap_y [height, 2], map_xy [2h, 2w, 2], map_frac [2h, 2w]) as the ingestion kernel reads them."""
+        w, h = self.cfg.width, self.cfg.height
+        tx = np.zeros((w, 2), np.int32); ty = np.zeros((h, 2), np.int32)
+        xy = np.zeros((2 * h, 2 * w, 2), np.int16); fr = np.zeros((2 * h, 2 * w), np.uint16)
+        self._chk(lib().ellc_read_camera_tables(self._h, _p(tx), _p(ty), _p(xy), _p(fr)))
+        return tx, ty, xy, fr
 
     def synchronize(self):
         self._chk(lib().ellc_synchronize(self._h))

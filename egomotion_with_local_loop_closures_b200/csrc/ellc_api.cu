@@ -117,6 +117,12 @@ struct ellc_handle {
     float* d_small;                                    // 128 floats in/out for solve_update
     float* d_weight; int64_t weight_cap;
     void* h_pin; void* d_pin; size_t pin_cap, pin_used;             // pinned bump arena for small H2D payloads
+    // camera ingestion (ellc_set_camera): resize taps, undistortion map at the tap positions, per-call job list, staging of host
+    // camera images; ingest_ev orders the copy stream -> ingest kernel (preparation stream) -> copy stream chain
+    bool cam_set; IngestGeo cam_geo;
+    int4* d_cam_cols; int4* d_cam_rows; uint2* d_cam_map; IngestJob* d_ingest_jobs;
+    uint8_t* d_cam_stage; size_t cam_stage_cap;
+    cudaEvent_t ingest_ev;
     std::string err;
     int64_t launches;
 };
@@ -204,10 +210,12 @@ int ellc_destroy(ellc_handle* h) {
     cudaFree(h->d_slots); cudaFree(h->d_slots_p); cudaFree(h->d_trace); cudaFree(h->d_small); cudaFree(h->d_eval_result); cudaFree(h->d_gen);
     for (int r = 0; r < 4; ++r) { cudaFree(h->d_pairs4[r]); cudaFree(h->d_results4[r]); cudaFree(h->d_order4[r]); cudaFree(h->d_gidx4[r]); }
     cudaFree(h->d_weight);
+    cudaFree(h->d_cam_cols); cudaFree(h->d_cam_rows); cudaFree(h->d_cam_map); cudaFree(h->d_ingest_jobs); cudaFree(h->d_cam_stage);
     if (h->h_pin) cudaFreeHost(h->h_pin);
     if (h->ev_valid) {
         for (int i = 0; i < 4; ++i) { cudaEventDestroy(h->ev0r[i]); cudaEventDestroy(h->ev1r[i]); }
         cudaEventDestroy(h->up_ev); cudaEventDestroy(h->prep_ev); cudaEventDestroy(h->main_ev); cudaEventDestroy(h->hyp_ev);
+        cudaEventDestroy(h->ingest_ev);
         for (int i = 0; i < 4; ++i) cudaEventDestroy(h->batch_ev[i]);
     }
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -279,6 +287,7 @@ int ellc_create(const ellc_config* cfg, ellc_handle** out) {
     CR_TRY(cudaEventCreateWithFlags(&h->prep_ev, cudaEventDisableTiming));
     CR_TRY(cudaEventCreateWithFlags(&h->main_ev, cudaEventDisableTiming));
     CR_TRY(cudaEventCreateWithFlags(&h->hyp_ev, cudaEventDisableTiming));
+    CR_TRY(cudaEventCreateWithFlags(&h->ingest_ev, cudaEventDisableTiming));
     for (int i = 0; i < 4; ++i) CR_TRY(cudaEventCreateWithFlags(&h->batch_ev[i], cudaEventDisableTiming));
     h->ev_valid = true;
     h->fr_reader.assign(cfg->max_frames, 0);
@@ -752,6 +761,150 @@ int ellc_upload_keyframe(ellc_handle* h, int32_t slot, const uint8_t* image, con
     h->kf_nvalid[slot] = -1;
     h->kf_dirty.push_back(slot);
     return after_upload(h);
+}
+
+int ellc_set_camera(ellc_handle* h, const ellc_camera* cam) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (!cam) { h->err = "null camera"; return ELLC_ERR_INVALID; }
+    const int W = h->cfg.width, H = h->cfg.height;
+    if ((cam->channels != 1 && cam->channels != 3) || (cam->undistort != 0 && cam->undistort != 1) || cam->width < W || cam->height < H ||
+        cam->width > 16384 || cam->height > 16384 || (int64_t)cam->pitch < (int64_t)cam->width * cam->channels) {
+        h->err = "unsupported camera (channels 1 or 3, undistort 0 or 1, working size <= camera size <= 16384, pitch >= width * channels)";
+        return ELLC_ERR_INVALID;
+    }
+    UndistortParams up;
+    std::memset(&up, 0, sizeof(up));
+    if (cam->undistort) {
+        for (int i = 0; i < 9; ++i) if (!std::isfinite(cam->K[i]) || !std::isfinite(cam->new_K[i])) { h->err = "non-finite camera matrix"; return ELLC_ERR_INVALID; }
+        for (int i = 0; i < 5; ++i) if (!std::isfinite(cam->dist[i])) { h->err = "non-finite distortion coefficient"; return ELLC_ERR_INVALID; }
+        if (!invert3(cam->new_K, up.ir)) { h->err = "singular new_K"; return ELLC_ERR_INVALID; }
+        up.fx = cam->K[0]; up.fy = cam->K[4]; up.u0 = cam->K[2]; up.v0 = cam->K[5];
+        up.k1 = cam->dist[0]; up.k2 = cam->dist[1]; up.p1 = cam->dist[2]; up.p2 = cam->dist[3]; up.k3 = cam->dist[4];
+    }
+    std::vector<int4> cols(W), rows(H);
+    build_resize_taps(cam->width, cam->height, W, H, cols.data(), rows.data());
+    CU_TRY(h, cudaSetDevice(h->cfg.device));
+    // the tables are read by ingestion kernels only (preparation stream), whose inputs come through the copy stream
+    CU_TRY(h, cudaStreamSynchronize(h->copy_stream));
+    CU_TRY(h, cudaStreamSynchronize(h->prep_stream));
+    if (!h->d_cam_cols) {
+        CU_TRY(h, cudaMalloc(&h->d_cam_cols, (size_t)W * sizeof(int4)));
+        CU_TRY(h, cudaMalloc(&h->d_cam_rows, (size_t)H * sizeof(int4)));
+        CU_TRY(h, cudaMalloc(&h->d_cam_map, (size_t)4 * W * H * sizeof(uint2)));
+        CU_TRY(h, cudaMalloc(&h->d_ingest_jobs, (size_t)h->slots_cap * sizeof(IngestJob)));
+    }
+    IngestGeo g = {cam->width, cam->height, cam->channels, cam->pitch, W, H, cam->undistort, 0};
+    CU_TRY(h, cudaMemcpyAsync(h->d_cam_cols, cols.data(), (size_t)W * sizeof(int4), cudaMemcpyHostToDevice, h->prep_stream));
+    CU_TRY(h, cudaMemcpyAsync(h->d_cam_rows, rows.data(), (size_t)H * sizeof(int4), cudaMemcpyHostToDevice, h->prep_stream));
+    if (cam->undistort) h->launches += launch_undistort_map(h->prep_stream, g, up, h->d_cam_cols, h->d_cam_rows, h->d_cam_map);
+    else CU_TRY(h, cudaMemsetAsync(h->d_cam_map, 0, (size_t)4 * W * H * sizeof(uint2), h->prep_stream));
+    CU_TRY(h, cudaGetLastError());
+    CU_TRY(h, cudaStreamSynchronize(h->prep_stream));       // cols / rows are host temporaries
+    h->cam_geo = g;
+    h->cam_set = true;
+    return ELLC_OK;
+}
+
+int ellc_read_camera_tables(ellc_handle* h, int32_t* tap_x, int32_t* tap_y, int16_t* map_xy, uint16_t* map_frac) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (!h->cam_set) { h->err = "no camera set (ellc_set_camera)"; return ELLC_ERR_NOT_READY; }
+    CU_TRY(h, cudaSetDevice(h->cfg.device));
+    const int W = h->cfg.width, H = h->cfg.height;
+    std::vector<int4> cols(W), rows(H);
+    std::vector<uint2> map((size_t)4 * W * H);
+    CU_TRY(h, cudaMemcpyAsync(cols.data(), h->d_cam_cols, (size_t)W * sizeof(int4), cudaMemcpyDeviceToHost, h->prep_stream));
+    CU_TRY(h, cudaMemcpyAsync(rows.data(), h->d_cam_rows, (size_t)H * sizeof(int4), cudaMemcpyDeviceToHost, h->prep_stream));
+    CU_TRY(h, cudaMemcpyAsync(map.data(), h->d_cam_map, map.size() * sizeof(uint2), cudaMemcpyDeviceToHost, h->prep_stream));
+    CU_TRY(h, cudaStreamSynchronize(h->prep_stream));
+    for (int i = 0; i < W; ++i) if (tap_x) { tap_x[2 * i] = cols[i].x; tap_x[2 * i + 1] = cols[i].y; }
+    for (int i = 0; i < H; ++i) if (tap_y) { tap_y[2 * i] = rows[i].x; tap_y[2 * i + 1] = rows[i].y; }
+    for (size_t i = 0; i < map.size(); ++i) {
+        if (map_xy) { map_xy[2 * i] = (int16_t)(map[i].x & 0xffffu); map_xy[2 * i + 1] = (int16_t)(map[i].x >> 16); }
+        if (map_frac) map_frac[i] = (uint16_t)map[i].y;
+    }
+    return ELLC_OK;
+}
+
+}  // extern "C"
+
+// n camera images -> level-0 images of n distinct slots of one pool.  Chain: copy stream (waits for the batches that read the
+// slots, guard_slot_write; copies host images into the staging buffer) -> ingest kernel on the preparation stream -> copy stream
+// (so that every consumer that waits for uploads, and the next staging copy, waits for the kernel too).
+static int ingest_impl(ellc_handle* h, int n, const int32_t* slots, const uint8_t* const* images, bool on_device, bool keyframe) {
+    const IngestGeo& g = h->cam_geo;
+    const size_t bytes = (size_t)g.pitch * (g.cam_h - 1) + (size_t)g.cam_w * g.channels, stride = (bytes + 255) & ~(size_t)255;
+    for (int i = 0; i < n; ++i) {
+        int rc = guard_slot_write(h, keyframe ? h->kf_reader[slots[i]] : h->fr_reader[slots[i]]);
+        if (rc) return rc;
+    }
+    std::vector<IngestJob> jobs(n);
+    uint8_t* pool = keyframe ? h->kf_img : h->fr_img;
+    for (int i = 0; i < n; ++i) jobs[i].dst = pool + (int64_t)slots[i] * h->geo.img_off[kLevels];
+    if (on_device) {
+        for (int i = 0; i < n; ++i) jobs[i].src = images[i];
+    } else {
+        if ((size_t)n * stride > h->cam_stage_cap) {       // the previous ingestion kernels may still read the old buffer
+            CU_TRY(h, cudaStreamSynchronize(h->copy_stream));
+            CU_TRY(h, cudaStreamSynchronize(h->prep_stream));
+            cudaFree(h->d_cam_stage); h->d_cam_stage = nullptr; h->cam_stage_cap = 0;
+            CU_TRY(h, cudaMalloc(&h->d_cam_stage, (size_t)n * stride));
+            h->cam_stage_cap = (size_t)n * stride;
+        }
+        for (int i = 0; i < n; ++i) {
+            jobs[i].src = h->d_cam_stage + (size_t)i * stride;
+            CU_TRY(h, cudaMemcpyAsync(h->d_cam_stage + (size_t)i * stride, images[i], bytes, cudaMemcpyHostToDevice, h->copy_stream));
+        }
+    }
+    CU_TRY(h, cudaEventRecord(h->ingest_ev, h->copy_stream));
+    CU_TRY(h, cudaStreamWaitEvent(h->prep_stream, h->ingest_ev, 0));
+    int rc = stage_h2d_on(h, h->prep_stream, h->d_ingest_jobs, jobs.data(), (size_t)n * sizeof(IngestJob));
+    if (rc) return rc;
+    h->launches += launch_ingest(h->prep_stream, h->d_ingest_jobs, n, g, h->d_cam_cols, h->d_cam_rows, h->d_cam_map);
+    CU_TRY(h, cudaGetLastError());
+    CU_TRY(h, cudaEventRecord(h->ingest_ev, h->prep_stream));
+    CU_TRY(h, cudaStreamWaitEvent(h->copy_stream, h->ingest_ev, 0));
+    for (int i = 0; i < n; ++i) {
+        const int s = slots[i];
+        if (keyframe) { h->kf_state[s] = 1; h->kf_lc_ready[s] = 0; h->kf_nvalid[s] = -1; h->kf_dirty.push_back(s); }
+        else { h->fr_state[s] = 1; h->fr_hist_ready[s] = 0; h->fr_dirty.push_back(s); }
+    }
+    return after_upload(h);
+}
+
+extern "C" {
+
+int ellc_ingest_frames(ellc_handle* h, int32_t n, const int32_t* slots, const uint8_t* const* images, int32_t on_device) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (n < 0 || n > h->cfg.max_frames || (n > 0 && (!slots || !images)) || (on_device != 0 && on_device != 1)) {
+        h->err = "bad frame slot list / image list"; return ELLC_ERR_INVALID;
+    }
+    std::vector<char> seen(h->cfg.max_frames, 0);
+    for (int i = 0; i < n; ++i) {
+        if (slots[i] < 0 || slots[i] >= h->cfg.max_frames || seen[slots[i]] || !images[i]) { h->err = "frame slot out of range / repeated, or null image"; return ELLC_ERR_INVALID; }
+        seen[slots[i]] = 1;
+    }
+    if (!h->cam_set) { h->err = "no camera set (ellc_set_camera)"; return ELLC_ERR_NOT_READY; }
+    if (n == 0) return ELLC_OK;
+    CU_TRY(h, cudaSetDevice(h->cfg.device));
+    return ingest_impl(h, n, slots, images, on_device == 1, false);
+}
+
+int ellc_ingest_keyframe(ellc_handle* h, int32_t slot, const uint8_t* image, int32_t on_device, const float* const depth[ELLC_LEVELS],
+                         const float* const var[ELLC_LEVELS]) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (!image || !depth || !var || slot < 0 || slot >= h->cfg.max_keyframes || (on_device != 0 && on_device != 1)) { h->err = "bad keyframe slot / null pointer"; return ELLC_ERR_INVALID; }
+    for (int l = 0; l < kLevels; ++l) if (!depth[l] || !var[l]) { h->err = "null depth/var level"; return ELLC_ERR_INVALID; }
+    if (!h->cam_set) { h->err = "no camera set (ellc_set_camera)"; return ELLC_ERR_NOT_READY; }
+    CU_TRY(h, cudaSetDevice(h->cfg.device));
+    int rc = guard_slot_write(h, h->kf_reader[slot]);
+    if (rc) return rc;
+    const int64_t win = h->geo.win_off[kLevels];
+    for (int l = 0; l < kLevels; ++l) {
+        const size_t bytes = (size_t)(h->geo.win_off[l + 1] - h->geo.win_off[l]) * sizeof(float);
+        CU_TRY(h, cudaMemcpyAsync(h->kf_depth + slot * win + h->geo.win_off[l], depth[l], bytes, cudaMemcpyHostToDevice, h->copy_stream));
+        CU_TRY(h, cudaMemcpyAsync(h->kf_var + slot * win + h->geo.win_off[l], var[l], bytes, cudaMemcpyHostToDevice, h->copy_stream));
+    }
+    return ingest_impl(h, 1, &slot, &image, on_device == 1, true);
 }
 
 int ellc_upload_keyframe_hypotheses(ellc_handle* h, int32_t slot, const uint8_t* image, const uint8_t* valid,

@@ -56,4 +56,15 @@ int launch_unzero_selftest(cudaStream_t st, long long n, unsigned long long seed
 int launch_invert6(cudaStream_t st, const float* d_in /*H36*/, float* d_out /*Hinv36 ok1*/);
 int launch_solve_update(cudaStream_t st, const float* d_in /*H36 b6 pose6 weight6*/, float* d_out /*pose6 delta6 wp1 ok1 rt12 small1*/, int fast);
 
+// ellc_ingest.cu -- camera frame -> level-0 image (gray, undistortion, resize in one pass)
+struct IngestJob { const uint8_t* src; uint8_t* dst; };                 // camera image (device), level-0 image of the slot
+struct IngestGeo { int cam_w, cam_h, channels, pitch, out_w, out_h, undistort, pad; };
+struct UndistortParams { double ir[9]; double fx, fy, u0, v0, k1, k2, p1, p2, k3; };
+// resize taps per output column / row: (source index 0, source index 1, Q11 coefficient 0, coefficient 1)
+int build_resize_taps(int cam_w, int cam_h, int out_w, int out_h, int4* cols, int4* rows);
+bool invert3(const double a[9], double b[9]);
+// map: (2 * out_h) x (2 * out_w) CV_16SC2 entries at the tap positions, (x | y << 16, frac)
+int launch_undistort_map(cudaStream_t st, const IngestGeo& g, const UndistortParams& p, const int4* d_cols, const int4* d_rows, uint2* d_map);
+int launch_ingest(cudaStream_t st, const IngestJob* d_jobs, int n, const IngestGeo& g, const int4* d_cols, const int4* d_rows, const uint2* d_map);
+
 }  // namespace ellc

@@ -18,6 +18,15 @@ extern int ORIG_COLS, ORIG_ROWS;                 // level-0 working size
 extern float ORIG_FX, ORIG_FY, ORIG_CX, ORIG_CY;
 void configure(int cols, int rows, float fx, float fy, float cx, float cy);
 
+// The camera of frame(camera_image, ...) (src/Frame.cpp:34-119): FLAG_DO_UNDISTORTION and DIM_FACTOR (RESIZE_FACTOR = 1 / DIM_FACTOR) of
+// src/ExternVariable.h, and the camera matrix / distortion coefficients the reference hands to cv::undistort.  configure_camera sets
+// ORIG_COLS / ORIG_ROWS to the camera size times RESIZE_FACTOR (rounded, as cv::resize sizes its output) and computes the
+// undistorted camera matrix with getOptimalNewCameraMatrix(K, dist, size, alpha) (ellc_optimal_new_camera_matrix).
+extern bool FLAG_DO_UNDISTORTION;
+extern float DIM_FACTOR;
+void configure_camera(int cam_cols, int cam_rows, int channels, const double K[9], const double dist[5], bool undistort,
+                      float dim_factor, double alpha);
+
 static const float weight[] = {100000.0f, 100000.0f, 100000.0f, 10000.0f, 10000.0f, 10000.0f};
 static const float CAMERA_PIXEL_NOISE_2 = 4.0f * 4.0f;
 static const float HUBER_D = 3.0f;

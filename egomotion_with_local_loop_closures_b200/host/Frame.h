@@ -18,6 +18,10 @@ public:
     // replaces frame(VideoCapture): the caller hands over the grayscale, undistorted, resized level-0 image
     // (src/Frame.cpp:45-75 is host I/O and stays with the caller)
     frame(const unsigned char* gray, int width, int height);
+    // what frame(VideoCapture) does after decoding: the camera image (BGR as VideoCapture delivers it, or 1 channel; rows
+    // contiguous) is converted to gray, undistorted (util::FLAG_DO_UNDISTORTION) and resized to ORIG_COLS x ORIG_ROWS on the GPU
+    // (util::configure_camera first)
+    frame(const unsigned char* camera_image, int cam_cols, int cam_rows, int channels);
     ~frame();
 
     int frameId;

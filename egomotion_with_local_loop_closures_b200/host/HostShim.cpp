@@ -43,6 +43,36 @@ int BATCH_SIZE = 0;
 void configure(int cols, int rows, float fx, float fy, float cx, float cy) {
     ORIG_COLS = cols; ORIG_ROWS = rows; ORIG_FX = fx; ORIG_FY = fy; ORIG_CX = cx; ORIG_CY = cy;
 }
+bool FLAG_DO_UNDISTORTION = false;
+float DIM_FACTOR = 4.0f;
+}  // namespace util
+
+namespace {
+ellc_camera g_camera;                           // util::configure_camera; applied to every context before its next ingestion
+unsigned long long g_camera_stamp = 0;
+std::mutex g_camera_mu;
+}  // namespace
+
+namespace util {
+void configure_camera(int cam_cols, int cam_rows, int channels, const double K[9], const double dist[5], bool undistort,
+                      float dim_factor, double alpha) {
+    ellc_camera cam;
+    std::memset(&cam, 0, sizeof(cam));
+    cam.width = cam_cols; cam.height = cam_rows; cam.channels = channels; cam.pitch = cam_cols * channels;
+    cam.undistort = undistort ? 1 : 0;
+    for (int i = 0; i < 9; ++i) cam.K[i] = K[i];
+    for (int i = 0; i < 5; ++i) cam.dist[i] = dist[i];
+    if (undistort && ellc_optimal_new_camera_matrix(K, dist, cam_cols, cam_rows, alpha, cam.new_K) != ELLC_OK)
+        throw std::runtime_error("configure_camera: invalid camera matrix / size");
+    FLAG_DO_UNDISTORTION = undistort;
+    DIM_FACTOR = dim_factor;
+    const double resize_factor = 1.0 / dim_factor;                      // RESIZE_FACTOR
+    ORIG_COLS = (int)std::lrint(cam_cols * resize_factor);                // cv::resize(src, dst, Size(), f, f): round(size * f)
+    ORIG_ROWS = (int)std::lrint(cam_rows * resize_factor);
+    std::lock_guard<std::mutex> lk(g_camera_mu);
+    g_camera = cam;
+    ++g_camera_stamp;
+}
 }  // namespace util
 
 namespace {
@@ -57,6 +87,7 @@ struct Context {
     std::vector<char> frame_pinned, kf_pinned;  // slots referenced by the batch being assembled: not evictable
     int next_frame = 0, next_kf = 0;
     int cols = 0, rows = 0;
+    unsigned long long camera_stamp = 0;        // g_camera_stamp last passed to ellc_set_camera
 };
 std::mutex g_registry_mu;
 std::vector<Context*> g_contexts;
@@ -100,6 +131,7 @@ Context* ctx() {
         c->kf_pinned.assign(kKfSlots, 0);
         c->next_frame = c->next_kf = 0;
         c->cols = util::ORIG_COLS; c->rows = util::ORIG_ROWS;
+        c->camera_stamp = 0;
     }
     return c;
 }
@@ -135,7 +167,23 @@ int take_slot(std::vector<frame*>& owner, std::vector<char>& pinned, int& next, 
     return -1;
 }
 
-int frame_slot(frame* f) {
+// util::configure_camera's camera on context c (before an ingestion)
+void apply_camera(Context* c) {
+    ellc_camera cam;
+    unsigned long long stamp;
+    {
+        std::lock_guard<std::mutex> lk(g_camera_mu);
+        cam = g_camera; stamp = g_camera_stamp;
+    }
+    if (stamp == 0) { t_err = "frame from a camera image: call util::configure_camera first"; throw std::runtime_error(t_err); }
+    if (c->camera_stamp == stamp) return;
+    if (ellc_set_camera(c->h, &cam) != ELLC_OK) fail("ellc_set_camera");
+    c->camera_stamp = stamp;
+}
+
+// the frame's slot in this thread's context; a frame that is not resident is uploaded from its image, or -- camera != NULL, at
+// construction -- ingested from the camera image
+int frame_slot(frame* f, const unsigned char* camera = nullptr) {
     Context* c = ctx();
     adopt(f, c);
     {
@@ -145,7 +193,12 @@ int frame_slot(frame* f) {
         if (s < 0) { t_err = "more distinct frames in one batch than frame slots"; throw std::runtime_error(t_err); }
         c->frame_owner[s] = f; f->gpu_frame_slot = s;
     }
-    if (ellc_upload_frame(c->h, f->gpu_frame_slot, f->image.ptr<uchar>(0)) != ELLC_OK) fail("ellc_upload_frame");
+    if (camera) {
+        apply_camera(c);
+        const int32_t s = f->gpu_frame_slot;
+        if (ellc_ingest_frames(c->h, 1, &s, &camera, 0) != ELLC_OK) fail("ellc_ingest_frames");
+        if (ellc_read_frame_level(c->h, s, 0, f->image.ptr<uchar>(0), nullptr, nullptr) != ELLC_OK) fail("ellc_read_frame_level");
+    } else if (ellc_upload_frame(c->h, f->gpu_frame_slot, f->image.ptr<uchar>(0)) != ELLC_OK) fail("ellc_upload_frame");
     return f->gpu_frame_slot;
 }
 
@@ -253,6 +306,7 @@ int context_count() {
 
 // ---- frame --------------------------------------------------------------------------------------------------------------
 int frame::numberOfInstances = 0;
+namespace { void finish_construction(frame* f); }
 
 frame::frame() : frameId(0), parentKeyframeId(0), isKeyframe(false), width(0), height(0), currentRows(0), currentCols(0),
                  pyrLevel(0), no_nonZeroDepthPts(0), rescaleFactor(1.0f), gpu_ctx(nullptr), gpu_frame_slot(-1), gpu_kf_slot(-1),
@@ -269,15 +323,38 @@ frame::frame(const unsigned char* gray, int w, int h) : frame() {
     width = w; height = h;
     image = Mat(h, w, ellc_host::CV_8UC1);
     std::memcpy(image.ptr<uchar>(0), gray, (size_t)w * h);
-    pyrLevel = 0; currentCols = w; currentRows = h;                          // :81-84
-    constructImagePyramids();                                                // :103
-    calculateGradient();                                                     // :104
-    depth = Mat::zeros(h, w, ellc_host::CV_32FC1);                            // :107-117
+    finish_construction(this);
+}
+
+// src/Frame.cpp:45-75 on the GPU: the level-0 image is built in the frame's slot and read back into `image`
+frame::frame(const unsigned char* camera_image, int cam_cols, int cam_rows, int channels) : frame() {
+    frameId = ++numberOfInstances;
+    {
+        std::lock_guard<std::mutex> lk(g_camera_mu);
+        if (g_camera_stamp == 0 || g_camera.width != cam_cols || g_camera.height != cam_rows || g_camera.channels != channels) {
+            t_err = "camera image does not match util::configure_camera"; throw std::runtime_error(t_err);
+        }
+    }
+    width = util::ORIG_COLS; height = util::ORIG_ROWS;
+    image = Mat(height, width, ellc_host::CV_8UC1);
+    frame_slot(this, camera_image);
+    finish_construction(this);
+}
+
+namespace {
+// the rest of frame::frame after the level-0 image exists (src/Frame.cpp:81-117)
+void finish_construction(frame* f) {
+    const int w = f->width, h = f->height;
+    f->pyrLevel = 0; f->currentCols = w; f->currentRows = h;                 // :81-84
+    f->constructImagePyramids();                                             // :103
+    f->calculateGradient();                                                  // :104
+    f->depth = Mat::zeros(h, w, ellc_host::CV_32FC1);                         // :107-117
     for (int l = 0; l < util::MAX_PYRAMID_LEVEL; ++l) {
-        depth_pyramid[l] = Mat::zeros(h >> l, w >> l, ellc_host::CV_32FC1);
-        weight_pyramid[l] = Mat::zeros(h >> l, w >> l, ellc_host::CV_32FC1);
+        f->depth_pyramid[l] = Mat::zeros(h >> l, w >> l, ellc_host::CV_32FC1);
+        f->weight_pyramid[l] = Mat::zeros(h >> l, w >> l, ellc_host::CV_32FC1);
     }
 }
+}  // namespace
 
 // `new frame(*currentframe)` (src/GlobalOptimize.cpp:181): member-wise copy -- cv::Mat members share their pixels, as in the
 // reference -- of a frame that is resident nowhere yet; weights accumulated on the device are pulled into the source's Mats
