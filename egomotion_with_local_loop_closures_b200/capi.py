@@ -12,6 +12,7 @@ import numpy as np
 LEVELS = 4
 MAX_TRACE_ITERS = 16
 ARITH_FAST, ARITH_STRICT = 0, 1
+ARITH_REFERENCE = 2        # STRICT + the reference's summation order and pose logarithm (bit-exact validation mode)
 PAIR_DEFAULT, PAIR_CONST_WEIGHT, PAIR_SAVE_WEIGHTS = 0, 1, 2
 _LIB_PATH = os.environ.get("ELLC_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "libellc_gn.so")
 
@@ -27,7 +28,7 @@ class Config(C.Structure):
                 ("weight", C.c_float * 6), ("stop_threshold", C.c_float), ("arithmetic", C.c_int32),
                 ("jacobian_at_warped", C.c_int32), ("max_keyframes", C.c_int32), ("max_frames", C.c_int32),
                 ("ctas_per_pair", C.c_int32), ("device", C.c_int32), ("pairs_per_cta", C.c_int32),
-                ("lm_lambda", C.c_float), ("lm_up", C.c_float), ("lm_down", C.c_float)]
+                ("lm_lambda", C.c_float), ("lm_up", C.c_float), ("lm_down", C.c_float), ("lc_bands", C.c_int32)]
 
 
 class Pair(C.Structure):

@@ -190,6 +190,7 @@ void ellc_default_config(ellc_config* c, int32_t width, int32_t height) {
     c->max_keyframes = 8; c->max_frames = 64;
     c->ctas_per_pair = 0; c->device = 0;
     c->lm_lambda = 0.0f; c->lm_up = 4.0f; c->lm_down = 0.5f;                              // 0 = the reference's plain Gauss-Newton step
+    c->lc_bands = 2;                                                                      // FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST
 }
 
 const char* ellc_last_error_string(const ellc_handle* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
@@ -237,6 +238,15 @@ int ellc_create(const ellc_config* cfg, ellc_handle** out) {
     }
     for (int l = 0; l < kLevels; ++l)
         if (cfg->max_iter[l] < 0) { g_create_err = "negative max_iter"; return ELLC_ERR_INVALID; }
+    if (cfg->arithmetic < ELLC_ARITH_FAST || cfg->arithmetic > ELLC_ARITH_REFERENCE) { g_create_err = "unknown arithmetic flavour"; return ELLC_ERR_INVALID; }
+    if (cfg->arithmetic == ELLC_ARITH_REFERENCE) {
+        // the reference's summation order is built for one CTA per pair, the PixelWisePyramid.cpp Jacobian and the plain step
+        if (cfg->jacobian_at_warped) { g_create_err = "ELLC_ARITH_REFERENCE does not cover the Pyramid.cpp variant (jacobian_at_warped)"; return ELLC_ERR_INVALID; }
+        if (cfg->lm_lambda != 0.0f) { g_create_err = "ELLC_ARITH_REFERENCE takes the reference's undamped step (lm_lambda = 0)"; return ELLC_ERR_INVALID; }
+        if (cfg->ctas_per_pair != 0 && cfg->ctas_per_pair != 1) { g_create_err = "ELLC_ARITH_REFERENCE tracks a pair on one CTA (ctas_per_pair 0 or 1)"; return ELLC_ERR_INVALID; }
+        if (cfg->pairs_per_cta != 0 && cfg->pairs_per_cta != 1) { g_create_err = "ELLC_ARITH_REFERENCE tracks one pair per CTA (pairs_per_cta 0 or 1)"; return ELLC_ERR_INVALID; }
+        if (cfg->lc_bands != 1 && cfg->lc_bands != 2) { g_create_err = "lc_bands must be 1 or 2"; return ELLC_ERR_INVALID; }
+    }
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev <= cfg->device) {
@@ -541,9 +551,11 @@ static void fill_params(const ellc_handle* h, TrackParams& p) {
     p.lm_lambda = h->cfg.lm_lambda > 0.f ? h->cfg.lm_lambda : 0.f;
     p.lm_up = h->cfg.lm_up > 1.f ? h->cfg.lm_up : 4.0f;
     p.lm_down = (h->cfg.lm_down > 0.f && h->cfg.lm_down <= 1.f) ? h->cfg.lm_down : 0.5f;
+    p.rowoff_pool = h->kf_rowoff; p.rows_total = h->rows_total; p.lc_bands = h->cfg.lc_bands;
 }
 
 static int pick_cluster(const ellc_handle* h, int n) {
+    if (h->cfg.arithmetic == ELLC_ARITH_REFERENCE) return 1;
     int c = h->cfg.ctas_per_pair;
     if (c == 1 || c == 2 || c == 4 || c == 8) return c;
     if (n >= 148) return 1;
@@ -555,7 +567,7 @@ static int pick_cluster(const ellc_handle* h, int n) {
 // Pairs per CTA (lockstep slots): with enough pairs to fill the GPU several times over, two pairs per CTA overlap their
 // serial solves; small batches keep one pair per CTA so that every SM gets work.
 static int pick_pairs_per_cta(const ellc_handle* h, int n, int cluster) {
-    if (cluster != 1) return 1;
+    if (cluster != 1 || h->cfg.arithmetic == ELLC_ARITH_REFERENCE) return 1;
     int np = h->cfg.pairs_per_cta;
     if (const char* e = std::getenv("ELLC_PAIRS_PER_CTA")) np = std::atoi(e);
     if (np >= 1 && np <= 4) return np;
@@ -699,13 +711,13 @@ static int track_launch(ellc_handle* h, int n, const ellc_pair* pairs, bool want
     if (const char* e = std::getenv("ELLC_DEBUG_MAX_ITER")) std::sscanf(e, "%d,%d,%d,%d", &p.max_iter[0], &p.max_iter[1], &p.max_iter[2], &p.max_iter[3]);
     if (const char* e = std::getenv("ELLC_DEBUG_NO_STOP")) if (*e == '1') p.stop_threshold = -1.0f;
     // Scheduling of the forward pairs: a cluster of CTAs per pair (few pairs: latency) or one CTA per 1..4 lockstep pairs
-    int l = launch_track(ts, p, cluster, h->cfg.arithmetic == ELLC_ARITH_STRICT);
+    int l = launch_track(ts, p, cluster, h->cfg.arithmetic);
     if (l < 0) { h->err = std::string("track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
     h->launches += l;
     if (n_fwd < n) {
         p.order = dev ? nullptr : h->d_order + n_fwd;
         p.n_pairs = n - n_fwd;
-        l = launch_track_lc(ts, p, h->cfg.arithmetic == ELLC_ARITH_STRICT);
+        l = launch_track_lc(ts, p, h->cfg.arithmetic);
         if (l < 0) { h->err = std::string("loop-closure track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
         h->launches += l;
     }
@@ -1293,13 +1305,14 @@ int ellc_gn_iterate(ellc_handle* h, int32_t kf_slot, int32_t frame_slot, int32_t
     fill_params(h, p);
     p.pairs = d_pair; p.results = h->d_eval_result; p.trace = h->d_trace; p.n_pairs = 1;
     p.level_hi = p.level_lo = level; p.iter_limit = 1; p.no_update = update ? 0 : 1;
-    // flavour: the handle's, except that the matrix-form Pyramid.cpp variant and the display planes exist in STRICT only
-    bool strict = h->cfg.arithmetic == ELLC_ARITH_STRICT;
-    if (variant == ELLC_VARIANT_PYRAMID) { strict = true; p.jacobian_at_warped = 1; }
+    // flavour: the handle's, except that the matrix-form Pyramid.cpp variant and the display planes exist in STRICT (and
+    // REFERENCE, which evaluates pixels as STRICT does) only
+    int arith = h->cfg.arithmetic;
+    if (variant == ELLC_VARIANT_PYRAMID) { arith = ELLC_ARITH_STRICT; p.jacobian_at_warped = 1; }
     if (variant == ELLC_VARIANT_FORWARD && !h->cfg.jacobian_at_warped) p.jacobian_at_warped = 0;
-    if (want_disp) { strict = true; p.disp_out = d_disp; }
+    if (want_disp) { if (arith == ELLC_ARITH_FAST) arith = ELLC_ARITH_STRICT; p.disp_out = d_disp; }
     p.weight_out = (weight_image || want_disp) ? h->d_weight : nullptr;
-    const int l = lc ? launch_track_lc(h->stream, p, strict) : launch_track(h->stream, p, pick_cluster(h, 1), strict);
+    const int l = lc ? launch_track_lc(h->stream, p, arith) : launch_track(h->stream, p, pick_cluster(h, 1), arith);
     if (l < 0) { h->err = std::string("track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
     h->launches += l;
     CU_TRY(h, cudaMemcpyAsync(out, h->d_trace + (int64_t)level * ELLC_MAX_TRACE_ITERS, sizeof(ellc_iter_trace), cudaMemcpyDeviceToHost, h->stream));
@@ -1345,7 +1358,7 @@ int ellc_solve_update_rt(ellc_handle* h, const float H[36], const float b[6], co
     for (int i = 0; i < 6; ++i) { in[36 + i] = b[i]; in[42 + i] = pose_in[i]; in[48 + i] = h->cfg.weight[i]; }
     int rc = stage_h2d(h, h->d_small, in, sizeof(in));
     if (rc) return rc;
-    h->launches += launch_solve_update(h->stream, h->d_small, h->d_small + 64, h->cfg.arithmetic == ELLC_ARITH_FAST ? 1 : 0);
+    h->launches += launch_solve_update(h->stream, h->d_small, h->d_small + 64, h->cfg.arithmetic);
     CU_TRY(h, cudaMemcpyAsync(outv, h->d_small + 64, sizeof(outv), cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
     for (int i = 0; i < 6; ++i) { pose_out[i] = outv[i]; delta[i] = outv[6 + i]; }
@@ -1559,7 +1572,8 @@ int ellc_prepare_keyframes_lc(ellc_handle* h, int32_t n, const int32_t* kf_slots
     rc = stage_h2d(h, d_slots, kf_slots, (size_t)n * sizeof(int));
     if (rc) return rc;
     h->launches += launch_lc_prepare(h->stream, h->kf_geo, h->kf_pix, h->geo.win_off[kLevels], h->kf_count, h->kf_img, h->geo.img_off[kLevels],
-                                     h->kf_weight, h->kf_lc, h->kf_lcf, h->kf_lcp, h->kf_lcH, h->K, d_slots, n, h->geo);
+                                     h->kf_weight, h->kf_lc, h->kf_lcf, h->kf_lcp, h->kf_lcH, h->K, d_slots, n, h->geo,
+                                     h->cfg.arithmetic == ELLC_ARITH_REFERENCE);
     CU_TRY(h, cudaGetLastError());
     for (int i = 0; i < n; ++i) h->kf_lc_ready[kf_slots[i]] = 1;
     return ELLC_OK;
@@ -1590,7 +1604,8 @@ int ellc_prepare_keyframes_lc_async(ellc_handle* h, int32_t n, const int32_t* kf
     rc = stage_h2d_on(h, h->prep_stream, d_slots, kf_slots, (size_t)n * sizeof(int));
     if (rc) return rc;
     h->launches += launch_lc_prepare(h->prep_stream, h->kf_geo, h->kf_pix, h->geo.win_off[kLevels], h->kf_count, h->kf_img, h->geo.img_off[kLevels],
-                                     h->kf_weight, h->kf_lc, h->kf_lcf, h->kf_lcp, h->kf_lcH, h->K, d_slots, n, h->geo);
+                                     h->kf_weight, h->kf_lc, h->kf_lcf, h->kf_lcp, h->kf_lcH, h->K, d_slots, n, h->geo,
+                                     h->cfg.arithmetic == ELLC_ARITH_REFERENCE);
     CU_TRY(h, cudaGetLastError());
     CU_TRY(h, cudaEventRecord(h->prep_ev, h->prep_stream));
     CU_TRY(h, cudaStreamWaitEvent(h->stream, h->prep_ev, 0));

@@ -122,6 +122,12 @@ struct TrackParams {
     int xchg_n;
     ellc_result* xchg_dst[ELLC_MAX_RANKS];
     const int* xchg_index;
+    // ELLC_ARITH_REFERENCE: the per-row record offsets of the selection lists ([kf_slot][rows_total], rows of the levels
+    // concatenated; select_scan_kernel), from which the row bands of the reference's summation become record ranges, and the
+    // number of row bands of the constant-weight variant (FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST ? 2 : 1)
+    const int* rowoff_pool;
+    int rows_total;
+    int lc_bands;
 };
 
 }  // namespace ellc

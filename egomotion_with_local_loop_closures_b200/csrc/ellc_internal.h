@@ -35,7 +35,8 @@ int launch_accumulate_weights(cudaStream_t st, float* kf_weight_slot, const uint
 int launch_finalise_weights(cudaStream_t st, float* kf_weight_slot, const int counts[kLevels], const Geometry& geo);
 int launch_lc_prepare(cudaStream_t st, const SelGeo* geo_pool, const SelPix* pix_pool, int64_t rec_slot_stride, const int* count_pool,
                       const uint8_t* img_pool, int64_t img_slot_stride, const float* weight_pool, LcRec* lc_pool, float4* lcf_pool,
-                      uint32_t* lcp_pool, float* lc_H, const LevelK* K, const int* d_slots, int n, const Geometry& geo);
+                      uint32_t* lcp_pool, float* lc_H, const LevelK* K, const int* d_slots, int n, const Geometry& geo,
+                      bool reference = false);   // reference: the hessian as ELLC_ARITH_REFERENCE sums it
 // dst (device, 4-byte aligned, capacity rounded up to 4 bytes) <- pinned host memory read by the SMs (no copy engine)
 int launch_fill_f32(cudaStream_t st, float* dst, float value, int64_t n);
 int launch_pull_host(cudaStream_t st, void* dst, const void* src_host_devptr, size_t bytes);
@@ -43,9 +44,9 @@ int launch_pull_host(cudaStream_t st, void* dst, const void* src_host_devptr, si
 // ellc_track.cu
 // Launches the GN tracking kernel for p.n_pairs pairs with `cluster` CTAs per pair.  Returns kernels launched (1) or a
 // negative value on launch-configuration failure (cudaGetLastError carries the reason).
-int launch_track(cudaStream_t st, const TrackParams& p, int cluster, bool strict);
+int launch_track(cudaStream_t st, const TrackParams& p, int cluster, int arithmetic);   // arithmetic: ELLC_ARITH_*
 // loop-closure (inverse-compositional constant-weight) variant: one CTA per pair, pairs = p.order[0 .. p.n_pairs)
-int launch_track_lc(cudaStream_t st, const TrackParams& p, bool strict);
+int launch_track_lc(cudaStream_t st, const TrackParams& p, int arithmetic);
 // result exchange: thread d adds n_records to *d_counters[d] (system scope)
 int launch_xchg_signal(cudaStream_t st, unsigned long long* const* d_counters, int n_dst, unsigned long long n_records);
 int launch_xchg_store(cudaStream_t st, unsigned long long* d_counter, unsigned long long value);
@@ -54,7 +55,7 @@ int launch_xchg_store(cudaStream_t st, unsigned long long* d_counter, unsigned l
 int launch_div_selftest(cudaStream_t st, long long n, unsigned long long seed, unsigned long long* d_counts /*[2]*/);
 int launch_unzero_selftest(cudaStream_t st, long long n, unsigned long long seed, unsigned long long* d_counts /*[1]*/);
 int launch_invert6(cudaStream_t st, const float* d_in /*H36*/, float* d_out /*Hinv36 ok1*/);
-int launch_solve_update(cudaStream_t st, const float* d_in /*H36 b6 pose6 weight6*/, float* d_out /*pose6 delta6 wp1 ok1 rt12 small1*/, int fast);
+int launch_solve_update(cudaStream_t st, const float* d_in /*H36 b6 pose6 weight6*/, float* d_out /*pose6 delta6 wp1 ok1 rt12 small1*/, int arithmetic);
 
 // ellc_ingest.cu -- camera frame -> level-0 image (gray, undistortion, resize in one pass)
 struct IngestJob { const uint8_t* src; uint8_t* dst; };                 // camera image (device), level-0 image of the slot

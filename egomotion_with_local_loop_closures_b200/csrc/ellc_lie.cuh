@@ -626,7 +626,39 @@ __device__ inline void delta_from_inverse_warp(const float (&col)[6], const floa
     for (int i = 1; i < 6; ++i) wp = ELLC_ADD(wp, fabsf(ELLC_MUL(delta[i], weight[i])));
     *weighted_pose = wp;
 }
-// pose <- log(exp(delta) exp(pose)) (:484) with the reference's Pade exponentials, lane-distributed
+// The logarithm of ELLC_ARITH_REFERENCE: the closed form of the oracle's rigid_log (oracle/ellc_oracle.cpp:181-203) operation for
+// operation -- every double operation individually rounded (no contraction), CUDA's double atan2 / sin / cos, the same
+// s < 1e-7 and theta < 1e-4 branches -- where se3_log_d takes power series below ~17 degrees.  The two agree to ~1e-16 before the
+// final rounding, but the closed form cancels at small angles (1 - cos theta), so only this one reproduces the reference's last
+// float bit of the translation.
+__device__ inline void m4_log_ref_f(const float (&T)[16], float out[6]) {
+    const double R00 = T[0], R01 = T[1], R02 = T[2];
+    const double R10 = T[4], R11 = T[5], R12 = T[6];
+    const double R20 = T[8], R21 = T[9], R22 = T[10];
+    const double t[3] = {T[3], T[7], T[11]};
+    const double ax = __dmul_rn(0.5, __dsub_rn(R21, R12)), ay = __dmul_rn(0.5, __dsub_rn(R02, R20)), az = __dmul_rn(0.5, __dsub_rn(R10, R01));
+    const double s = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(ax, ax), __dmul_rn(ay, ay)), __dmul_rn(az, az)));
+    const double c = __dmul_rn(0.5, __dsub_rn(__dadd_rn(__dadd_rn(R00, R11), R22), 1.0));
+    const double th = atan2(s, c);
+    double k;
+    if (s < 1e-7) k = (c > 0) ? __dadd_rn(1.0, __ddiv_rn(__dmul_rn(th, th), 6.0)) : 0.0;
+    else k = __ddiv_rn(th, s);
+    const double w[3] = {__dmul_rn(k, ax), __dmul_rn(k, ay), __dmul_rn(k, az)};
+    double coef;
+    if (th < 1e-4) coef = __dadd_rn(1.0 / 12.0, __ddiv_rn(__dmul_rn(th, th), 720.0));
+    else coef = __ddiv_rn(__dsub_rn(1.0, __ddiv_rn(__dmul_rn(th, sin(th)), __dmul_rn(2.0, __dsub_rn(1.0, cos(th))))), __dmul_rn(th, th));
+    const double wt[3] = {__dsub_rn(__dmul_rn(w[1], t[2]), __dmul_rn(w[2], t[1])), __dsub_rn(__dmul_rn(w[2], t[0]), __dmul_rn(w[0], t[2])),
+                          __dsub_rn(__dmul_rn(w[0], t[1]), __dmul_rn(w[1], t[0]))};
+    const double wwt[3] = {__dsub_rn(__dmul_rn(w[1], wt[2]), __dmul_rn(w[2], wt[1])), __dsub_rn(__dmul_rn(w[2], wt[0]), __dmul_rn(w[0], wt[2])),
+                           __dsub_rn(__dmul_rn(w[0], wt[1]), __dmul_rn(w[1], wt[0]))};
+    out[0] = (float)w[0]; out[1] = (float)w[1]; out[2] = (float)w[2];
+    ELLC_UNROLL
+    for (int i = 0; i < 3; ++i) out[3 + i] = (float)__dadd_rn(__dsub_rn(t[i], __dmul_rn(0.5, wt[i])), __dmul_rn(coef, wwt[i]));
+}
+
+// pose <- log(exp(delta) exp(pose)) (:484) with the reference's Pade exponentials, lane-distributed; REF: the logarithm in the
+// oracle's closed form (m4_log_ref_f)
+template <bool REF = false>
 __device__ inline void pose_update_pade_warp(const float (&delta)[6], float rt_pose_e, float (&pose)[6], float* rt_new_e, int lane) {
     const int e = lane & 15;
     const float Ta = se3_exp_pade_warp(delta[0], delta[1], delta[2], delta[3], delta[4], delta[5], e);
@@ -635,7 +667,8 @@ __device__ inline void pose_update_pade_warp(const float (&delta)[6], float rt_p
     ELLC_UNROLL
     for (int i = 0; i < 12; ++i) T[i] = __shfl_sync(kFullWarp, Te, i);
     T[12] = T[13] = T[14] = 0.f; T[15] = 1.f;                  // not read by the logarithm
-    m4_log_f(T, pose);
+    if constexpr (REF) m4_log_ref_f(T, pose);
+    else m4_log_f(T, pose);
     *rt_new_e = se3_exp_pade_warp(pose[0], pose[1], pose[2], pose[3], pose[4], pose[5], e);
 }
 // updatePose() given column (lane % 6) of hessianInv in col[0..5]

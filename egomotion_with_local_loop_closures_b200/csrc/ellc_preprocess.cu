@@ -368,6 +368,9 @@ __global__ void __launch_bounds__(256) finalise_weights_kernel(float* __restrict
 // double and rounds once, so the sum is taken in double here too (the order of a double sum of ~1e5 float products does not
 // reach the fp32 result).  One CTA per (level, keyframe); the Jacobian follows the reference's operation sequence exactly
 // (fp32, with the sub-expressions C++ promotes to double through pow()).
+// REF (ELLC_ARITH_REFERENCE): the reference's own order instead of the tree -- thread a*6+b sums (double)(J_a w) * (double)J_b over
+// the level's records in raster order, one double addition after the other from +0 (the products are exact), and rounds once.
+template <bool REF>
 __global__ void __launch_bounds__(256)
 lc_prepare_kernel(const SelGeo* __restrict__ geo_pool, const SelPix* __restrict__ pix_pool, int64_t rec_slot_stride,
                   const int* __restrict__ count_pool, const uint8_t* __restrict__ img_pool, int64_t img_slot_stride,
@@ -424,28 +427,41 @@ lc_prepare_kernel(const SelGeo* __restrict__ geo_pool, const SelPix* __restrict_
         // DRAM every iteration (the records of the resident keyframes are far larger than L2)
         lcf_pool[rec_off + i] = make_float4(sg.wX, sg.wY, sg.depth, rec.w);
         lcp_pool[rec_off + i] = (uint32_t)(gx2 + 512) | ((uint32_t)(gy2 + 512) << 10) | ((uint32_t)c << 24);
+        if constexpr (!REF) {
 #pragma unroll
-        for (int a = 0; a < 6; ++a) {
-            const double wj = (double)__fmul_rn(rec.J[a], rec.w);                      // weightedSteepestDescent :668-673
+            for (int a = 0; a < 6; ++a) {
+                const double wj = (double)__fmul_rn(rec.J[a], rec.w);                  // weightedSteepestDescent :668-673
 #pragma unroll
-            for (int b = 0; b < 6; ++b) Hd[a * 6 + b] = fma(wj, (double)rec.J[b], Hd[a * 6 + b]);
+                for (int b = 0; b < 6; ++b) Hd[a * 6 + b] = fma(wj, (double)rec.J[b], Hd[a * 6 + b]);
+            }
         }
     }
     __shared__ double s_part[8][36];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if constexpr (!REF) {
 #pragma unroll
-    for (int i = 0; i < 36; ++i) {
-        double v = Hd[i];
+        for (int i = 0; i < 36; ++i) {
+            double v = Hd[i];
 #pragma unroll
-        for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (lane == 0) s_part[warp][i] = v;
+            for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            if (lane == 0) s_part[warp][i] = v;
+        }
     }
-    __syncthreads();
+    __syncthreads();                                                                   // (REF: the level's records are written)
     __shared__ float s_H[36];
     float* const rec = lc_H + ((int64_t)slot * kLevels + level) * kLcHStride;
     if (threadIdx.x < 36) {
-        double t = s_part[0][threadIdx.x];
-        for (int w = 1; w < 8; ++w) t += s_part[w][threadIdx.x];
+        double t;
+        if constexpr (REF) {
+            const int a = threadIdx.x / 6, b = threadIdx.x % 6;
+            const LcRec* lr = lc_pool + rec_off;
+            t = 0.0;
+#pragma unroll 4
+            for (int i = 0; i < n; ++i) t = __dadd_rn(t, __dmul_rn((double)__fmul_rn(lr[i].J[a], lr[i].w), (double)lr[i].J[b]));
+        } else {
+            t = s_part[0][threadIdx.x];
+            for (int w = 1; w < 8; ++w) t += s_part[w][threadIdx.x];
+        }
         s_H[threadIdx.x] = (float)t;
         rec[threadIdx.x] = (float)t;
     }
@@ -660,11 +676,15 @@ int launch_finalise_weights(cudaStream_t st, float* kf_weight_slot, const int co
 
 int launch_lc_prepare(cudaStream_t st, const SelGeo* geo_pool, const SelPix* pix_pool, int64_t rec_slot_stride, const int* count_pool,
                       const uint8_t* img_pool, int64_t img_slot_stride, const float* weight_pool, LcRec* lc_pool, float4* lcf_pool,
-                      uint32_t* lcp_pool, float* lc_H, const LevelK* K, const int* d_slots, int n, const Geometry& geo) {
+                      uint32_t* lcp_pool, float* lc_H, const LevelK* K, const int* d_slots, int n, const Geometry& geo, bool reference) {
     KSet ks;
     for (int l = 0; l < kLevels; ++l) ks.k[l] = K[l];
-    lc_prepare_kernel<<<dim3(kLevels, n), 256, 0, st>>>(geo_pool, pix_pool, rec_slot_stride, count_pool, img_pool, img_slot_stride,
-                                                        weight_pool, lc_pool, lcf_pool, lcp_pool, lc_H, ks, d_slots, geo);
+    if (reference)
+        lc_prepare_kernel<true><<<dim3(kLevels, n), 256, 0, st>>>(geo_pool, pix_pool, rec_slot_stride, count_pool, img_pool, img_slot_stride,
+                                                                  weight_pool, lc_pool, lcf_pool, lcp_pool, lc_H, ks, d_slots, geo);
+    else
+        lc_prepare_kernel<false><<<dim3(kLevels, n), 256, 0, st>>>(geo_pool, pix_pool, rec_slot_stride, count_pool, img_pool, img_slot_stride,
+                                                                   weight_pool, lc_pool, lcf_pool, lcp_pool, lc_H, ks, d_slots, geo);
     return 1;
 }
 

@@ -36,6 +36,12 @@ extern int MAX_ITER[4];                          // src/main.cpp:34
 extern bool FLAG_DO_PARALLEL_POSE_ESTIMATION;    // must stay true: this shim IS that path
 extern bool FLAG_INITIALIZE_NONZERO_POSE;
 extern bool FLAG_DO_CONST_WEIGHT_POSE_ESTIMATION;
+extern bool FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST;  // constant-weight tracks sum over two row bands (src/PixelWisePyramid.cpp:945-951)
+                                                 // instead of one (:970); read by ELLC_ARITH_REFERENCE only (ellc_config::lc_bands)
+// Arithmetic flavour of the GPU tracker (ELLC_ARITH_FAST, ELLC_ARITH_STRICT or ELLC_ARITH_REFERENCE of ellc_gn.h; default FAST).
+// ELLC_ARITH_REFERENCE reproduces the reference's tracker bit for bit, so that poses_orig.txt / matchframes*.txt of a run can be
+// diffed against a CPU run of the reference.  Read when a thread's context creates its tracker (and again after a change).
+extern int GPU_ARITHMETIC;
 extern bool FLAG_DO_LOOP_CLOSURE;
 extern bool FLAG_ALTERNATE_GN_RA;                // batch alternation with rotation averaging ("LC" mode, src/main.cpp:89-92)
 extern bool FLAG_IS_BOOTSTRAP;

@@ -35,6 +35,8 @@ int MAX_ITER[4] = {4, 7, 9, 12};
 bool FLAG_DO_PARALLEL_POSE_ESTIMATION = true;
 bool FLAG_INITIALIZE_NONZERO_POSE = false;
 bool FLAG_DO_CONST_WEIGHT_POSE_ESTIMATION = false;
+bool FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST = true;
+int GPU_ARITHMETIC = ELLC_ARITH_FAST;
 bool FLAG_DO_LOOP_CLOSURE = false;
 bool FLAG_ALTERNATE_GN_RA = false;
 bool FLAG_IS_BOOTSTRAP = false;
@@ -87,6 +89,7 @@ struct Context {
     std::vector<char> frame_pinned, kf_pinned;  // slots referenced by the batch being assembled: not evictable
     int next_frame = 0, next_kf = 0;
     int cols = 0, rows = 0;
+    int arithmetic = 0, lc_bands = 0;           // util::GPU_ARITHMETIC / FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST the tracker was built with
     unsigned long long camera_stamp = 0;        // g_camera_stamp last passed to ellc_set_camera
 };
 std::mutex g_registry_mu;
@@ -107,7 +110,8 @@ Context* ctx() {
         g_contexts.push_back(c);
         t_ctx = c;
     }
-    if (c->h && (c->cols != util::ORIG_COLS || c->rows != util::ORIG_ROWS)) {
+    const int lc_bands = util::FLAG_DO_PARALLEL_CONST_WEIGHT_POSE_EST ? 2 : 1;
+    if (c->h && (c->cols != util::ORIG_COLS || c->rows != util::ORIG_ROWS || c->arithmetic != util::GPU_ARITHMETIC || c->lc_bands != lc_bands)) {
         std::lock_guard<std::mutex> lk(c->table_mu);
         for (frame* f : c->frame_owner) if (f && f->gpu_ctx == c) f->gpu_frame_slot = -1;
         for (frame* f : c->kf_owner) if (f && f->gpu_ctx == c) { f->gpu_kf_slot = -1; f->gpu_lc_ready = false; }
@@ -122,6 +126,8 @@ Context* ctx() {
         cfg.huber_d = util::HUBER_D; cfg.camera_pixel_noise_2 = util::CAMERA_PIXEL_NOISE_2;
         for (int i = 0; i < 6; ++i) cfg.weight[i] = util::weight[i];
         cfg.max_frames = kFrameSlots; cfg.max_keyframes = kKfSlots;
+        cfg.arithmetic = util::GPU_ARITHMETIC;
+        cfg.lc_bands = lc_bands;
         if (ellc_create(&cfg, &c->h) != ELLC_OK) fail("ellc_create");
         std::lock_guard<std::mutex> lk(c->table_mu);
         c->frame_owner.assign(kFrameSlots, nullptr);
@@ -131,6 +137,7 @@ Context* ctx() {
         c->kf_pinned.assign(kKfSlots, 0);
         c->next_frame = c->next_kf = 0;
         c->cols = util::ORIG_COLS; c->rows = util::ORIG_ROWS;
+        c->arithmetic = util::GPU_ARITHMETIC; c->lc_bands = lc_bands;
         c->camera_stamp = 0;
     }
     return c;
