@@ -50,11 +50,11 @@ int launch_track_lc(cudaStream_t st, const TrackParams& p, int arithmetic);
 // result exchange: thread d adds n_records to *d_counters[d] (system scope)
 int launch_xchg_signal(cudaStream_t st, unsigned long long* const* d_counters, int n_dst, unsigned long long n_records);
 int launch_xchg_store(cudaStream_t st, unsigned long long* d_counter, unsigned long long value);
-// single-thread kernel running solve_update_f on the device (ellc_solve_update)
 // div2_rn_shared (the pixel loop's shared-reciprocal exact division) against __fdiv_rn on n pseudo-random operand triples
 int launch_div_selftest(cudaStream_t st, long long n, unsigned long long seed, unsigned long long* d_counts /*[2]*/);
 int launch_unzero_selftest(cudaStream_t st, long long n, unsigned long long seed, unsigned long long* d_counts /*[1]*/);
 int launch_invert6(cudaStream_t st, const float* d_in /*H36*/, float* d_out /*Hinv36 ok1*/);
+// one-warp kernel running K5's LU, deltapose / weightedPose and pose update of the given flavour (ellc_solve_update)
 int launch_solve_update(cudaStream_t st, const float* d_in /*H36 b6 pose6 weight6*/, float* d_out /*pose6 delta6 wp1 ok1 rt12 small1*/, int arithmetic);
 
 // ellc_ingest.cu -- camera frame -> level-0 image (gray, undistortion, resize in one pass)
