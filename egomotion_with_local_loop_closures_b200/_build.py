@@ -5,7 +5,7 @@ import subprocess
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libellc_gn.so")
-SOURCES = ["ellc_api.cu", "ellc_preprocess.cu", "ellc_track.cu", "ellc_ingest.cu"]
+SOURCES = ["ellc_api.cu", "ellc_preprocess.cu", "ellc_track.cu", "ellc_ingest.cu", "ellc_sequence.cu"]
 HEADERS = ["ellc_common.cuh", "ellc_internal.h", "ellc_lie.cuh", os.path.join("..", "..", "include", "ellc_gn.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC,-ffp-contract=off", "-shared"]

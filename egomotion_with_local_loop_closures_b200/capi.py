@@ -50,6 +50,11 @@ class IterTrace(C.Structure):
                 ("pad", C.c_int32 * 3)]
 
 
+class SeqStep(C.Structure):
+    _fields_ = [("kf_slot", C.c_int32), ("frame_slot", C.c_int32), ("prev_step", C.c_int32), ("kf_step", C.c_int32),
+                ("prev_world", C.c_float * 6), ("kf_world", C.c_float * 6), ("flags", C.c_int32), ("reserved", C.c_int32)]
+
+
 class Camera(C.Structure):
     _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("channels", C.c_int32), ("pitch", C.c_int32),
                 ("undistort", C.c_int32), ("reserved", C.c_int32), ("K", C.c_double * 9), ("dist", C.c_double * 5),
@@ -72,7 +77,10 @@ LC_RING_DTYPE = np.dtype([("frame_id", "<i4"), ("is_valid", "<i4"), ("frame_slot
 LC_QUERY_DTYPE = np.dtype([("current_array_id", "<i4"), ("match_window_beg", "<i4"), ("match_window_end", "<i4"), ("frame_id", "<i4"),
                            ("frame_slot", "<i4"), ("stray", "<i4"), ("pose_world", "<f4", 6)])
 assert LC_CAND_DTYPE.itemsize == 56 and LC_STATS_DTYPE.itemsize == 24 and LC_RING_DTYPE.itemsize == 40 and LC_QUERY_DTYPE.itemsize == 48
+SEQ_STEP_DTYPE = np.dtype([("kf_slot", "<i4"), ("frame_slot", "<i4"), ("prev_step", "<i4"), ("kf_step", "<i4"),
+                           ("prev_world", "<f4", 6), ("kf_world", "<f4", 6), ("flags", "<i4"), ("reserved", "<i4")])
 assert PAIR_DTYPE.itemsize == 36 and RESULT_DTYPE.itemsize == 256 and TRACE_DTYPE.itemsize == 256
+assert C.sizeof(SeqStep) == SEQ_STEP_DTYPE.itemsize == 72
 
 # every symbol include/ellc_gn.h declares
 SYMBOLS = ["ellc_default_config", "ellc_create", "ellc_destroy", "ellc_last_error_string", "ellc_version",
@@ -88,7 +96,8 @@ SYMBOLS = ["ellc_default_config", "ellc_create", "ellc_destroy", "ellc_last_erro
            "ellc_exchange_create", "ellc_exchange_attach_ipc", "ellc_exchange_attach_local", "ellc_track_batch_exchange",
            "ellc_exchange_wait", "ellc_exchange_destroy", "ellc_se3_exp_closed", "ellc_se3_log_closed",
            "ellc_gn_iterate", "ellc_hessian_inverse", "ellc_lc_generate_pairs", "ellc_track_generated_pairs",
-           "ellc_optimal_new_camera_matrix", "ellc_set_camera", "ellc_ingest_frames", "ellc_ingest_keyframe", "ellc_read_camera_tables"]
+           "ellc_optimal_new_camera_matrix", "ellc_set_camera", "ellc_ingest_frames", "ellc_ingest_keyframe", "ellc_read_camera_tables",
+           "ellc_track_sequence_steps"]
 VARIANT_FORWARD, VARIANT_CONST_WEIGHT, VARIANT_PYRAMID = 0, 1, 2
 
 
@@ -183,6 +192,7 @@ def lib():
         L.ellc_ingest_keyframe.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
         L.ellc_read_camera_tables.argtypes = [C.c_void_p] + [C.c_void_p] * 4
         L.ellc_se3_log_closed.argtypes = [C.c_void_p] * 2
+        L.ellc_track_sequence_steps.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -407,6 +417,33 @@ class Tracker:
         self._chk(lib().ellc_track_batch(self._h, n, _p(pairs), _p(res), _p(tr)))
         self._keep = []
         return (res, tr) if want_trace else res
+
+    @staticmethod
+    def make_steps(kf_slots, frame_slots, prev_steps, kf_steps, prev_world=None, kf_world=None, flags=0):
+        """An ellc_seq_step array; prev_world / kf_world (n x 6) are only read where prev_steps / kf_steps are -1."""
+        n = len(kf_slots)
+        steps = np.zeros(n, SEQ_STEP_DTYPE)
+        steps["kf_slot"] = kf_slots
+        steps["frame_slot"] = frame_slots
+        steps["prev_step"] = prev_steps
+        steps["kf_step"] = kf_steps
+        if prev_world is not None:
+            steps["prev_world"] = np.asarray(prev_world, np.float32).reshape(n, 6)
+        if kf_world is not None:
+            steps["kf_world"] = np.asarray(kf_world, np.float32).reshape(n, 6)
+        steps["flags"] = flags
+        return steps
+
+    def track_sequence_steps(self, steps):
+        """Track frame sequences with the pose chain on the device (ellc_track_sequence_steps).  Returns (results, world): the
+        ellc_result records and the world poses (n x 6 float32) of the steps, in input order."""
+        steps = np.ascontiguousarray(steps, SEQ_STEP_DTYPE)
+        n = len(steps)
+        res = np.zeros(n, RESULT_DTYPE)
+        world = np.zeros((n, 6), np.float32)
+        self._chk(lib().ellc_track_sequence_steps(self._h, n, _p(steps), _p(res), _p(world)))
+        self._keep = []
+        return res, world
 
     def track_batch_async(self, pairs):
         pairs = np.ascontiguousarray(pairs, PAIR_DTYPE)

@@ -114,6 +114,7 @@ struct ellc_handle {
     ellc_pair* d_gen_pairs; int gen_n, gen_flags;
     std::vector<int> gen_kf_slots, gen_frame_slots;    // slots the generated pairs may read (slot-reuse bookkeeping)
     ellc_iter_trace* d_trace; int64_t trace_cap;
+    char* d_seq; size_t seq_bytes;                     // buffer of ellc_track_sequence_steps (steps, order, pairs, records, world poses)
     float* d_small;                                    // 128 floats in/out for solve_update
     float* d_weight; int64_t weight_cap;
     void* h_pin; void* d_pin; size_t pin_cap, pin_used;             // pinned bump arena for small H2D payloads
@@ -209,6 +210,7 @@ int ellc_destroy(ellc_handle* h) {
     cudaFree(h->d_hyp); cudaFree(h->d_nvalid); cudaFree(h->fr_hist);
     cudaFree(h->fr_weight); cudaFree(h->kf_weight); cudaFree(h->kf_lc); cudaFree(h->kf_lcH); cudaFree(h->kf_lcf); cudaFree(h->kf_lcp); cudaFree(h->kf_count); cudaFree(h->kf_rowcount); cudaFree(h->kf_rowoff);
     cudaFree(h->d_slots); cudaFree(h->d_slots_p); cudaFree(h->d_trace); cudaFree(h->d_small); cudaFree(h->d_eval_result); cudaFree(h->d_gen);
+    cudaFree(h->d_seq);
     for (int r = 0; r < 4; ++r) { cudaFree(h->d_pairs4[r]); cudaFree(h->d_results4[r]); cudaFree(h->d_order4[r]); cudaFree(h->d_gidx4[r]); }
     cudaFree(h->d_weight);
     cudaFree(h->d_cam_cols); cudaFree(h->d_cam_rows); cudaFree(h->d_cam_map); cudaFree(h->d_ingest_jobs); cudaFree(h->d_cam_stage);
@@ -606,6 +608,37 @@ static int xchg_publish(ellc_handle* h, cudaStream_t st) {
     return ELLC_OK;
 }
 
+// Bookkeeping every tracking call shares (ellc_track_batch*, ellc_track_sequence_steps).  batch_begin numbers the batch; its
+// completion event batch_ev[seq & 3] and timing events ev0r / ev1r are those of batch seq - 4, which is waited for first (ring of
+// 4).
+static int batch_begin(ellc_handle* h, long long* seq_out) {
+    const long long seq = h->batch_seq + 1;
+    if (seq > 4 && seq - 4 > h->batch_done_seq) {
+        CU_TRY(h, cudaEventSynchronize(h->batch_ev[seq & 3]));
+        if (seq - 4 > h->batch_done_seq) h->batch_done_seq = seq - 4;          // batches complete in order of their streams' events
+    }
+    *seq_out = seq;
+    return ELLC_OK;
+}
+// Ordering of the batch's stream: behind everything enqueued on the main stream so far (synchronous preparation, weight
+// and loop-closure kernels, and -- through the main stream's wait on prep_ev -- the pipelined preparation); NOT behind the
+// previous batch, which runs on the other tracking stream, unless this batch shares buffers with it (serial: trace, weight images).
+static int batch_order(ellc_handle* h, long long seq, bool serial) {
+    cudaStream_t ts = h->tstream[seq & 1];
+    CU_TRY(h, cudaEventRecord(h->main_ev, h->stream));
+    CU_TRY(h, cudaStreamWaitEvent(ts, h->main_ev, 0));
+    if (serial && seq > 1 && seq - 1 > h->batch_done_seq) CU_TRY(h, cudaStreamWaitEvent(ts, h->batch_ev[(seq - 1) & 3], 0));
+    return xchg_publish(h, ts);                            // tables this rank has copied out since its last batch: tell the senders
+}
+// The batch's kernels are enqueued: its completion event, after which it is the last batch
+static int batch_end(ellc_handle* h, long long seq) {
+    cudaStream_t ts = h->tstream[seq & 1];
+    CU_TRY(h, cudaEventRecord(h->ev1r[seq & 3], ts));
+    CU_TRY(h, cudaEventRecord(h->batch_ev[seq & 3], ts));
+    h->batch_seq = seq;
+    return ELLC_OK;
+}
+
 // Launch parameters of the optional result exchange of a batch (ellc_track_batch_exchange)
 struct XchgLaunch {
     int n_dst = 0;
@@ -629,13 +662,11 @@ static int track_launch(ellc_handle* h, int n, const ellc_pair* pairs, bool want
     rc = flush_dirty(h);
     if (rc) return rc;
     // batch bookkeeping: sequence number, ring entry (staging + result buffers: a finished batch can be downloaded while the next two
-    // run), completion event (ring of 4: reusing an entry requires its old batch to be finished)
-    const long long seq = h->batch_seq + 1;
+    // run), completion event
+    long long seq = 0;
+    rc = batch_begin(h, &seq);
+    if (rc) return rc;
     const int r = (int)(seq & 3);
-    if (seq > 4 && seq - 4 > h->batch_done_seq) {
-        CU_TRY(h, cudaEventSynchronize(h->batch_ev[r]));
-        if (seq - 4 > h->batch_done_seq) h->batch_done_seq = seq - 4;          // batches complete in order of their streams' events
-    }
     rc = ensure_ring_cap(h, r, n, want_trace);
     if (rc) return rc;
     h->d_pairs = h->d_pairs4[r]; h->d_order = h->d_order4[r]; h->d_results = h->d_results4[r];
@@ -673,14 +704,7 @@ static int track_launch(ellc_handle* h, int n, const ellc_pair* pairs, bool want
         rc = ensure_lc_pools(h);
         if (rc) return rc;
     }
-    // Ordering of the batch's stream: behind everything enqueued on the main stream so far (synchronous preparation, weight
-    // and loop-closure kernels, and -- through the main stream's wait on prep_ev -- the pipelined preparation); NOT behind the
-    // previous batch, which runs on the other tracking stream, unless this batch shares buffers with it (trace, weight images).
-    CU_TRY(h, cudaEventRecord(h->main_ev, h->stream));
-    CU_TRY(h, cudaStreamWaitEvent(ts, h->main_ev, 0));
-    const bool serial = !h->overlap_batches || want_trace || save_weights || n_fwd < n;
-    if (serial && seq > 1 && seq - 1 > h->batch_done_seq) CU_TRY(h, cudaStreamWaitEvent(ts, h->batch_ev[(seq - 1) & 3], 0));
-    rc = xchg_publish(h, ts);                              // tables this rank has copied out since its last batch: tell the senders
+    rc = batch_order(h, seq, !h->overlap_batches || want_trace || save_weights || n_fwd < n);
     if (rc) return rc;
     if (!dev) {
         rc = stage_h2d_on(h, ts, h->d_pairs, pairs, (size_t)n * sizeof(ellc_pair));
@@ -721,9 +745,8 @@ static int track_launch(ellc_handle* h, int n, const ellc_pair* pairs, bool want
         if (l < 0) { h->err = std::string("loop-closure track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
         h->launches += l;
     }
-    CU_TRY(h, cudaEventRecord(h->ev1r[r], ts));
-    CU_TRY(h, cudaEventRecord(h->batch_ev[r], ts));
-    h->batch_seq = seq;
+    rc = batch_end(h, seq);
+    if (rc) return rc;
     h->res_seq[r] = seq;
     h->res_taken[r] = xl != nullptr;                       // exchanged batches are read from the exchange tables, not from this buffer
     if (dev) {
@@ -1256,6 +1279,117 @@ int ellc_track_batch(ellc_handle* h, int32_t n, const ellc_pair* pairs, ellc_res
     CU_TRY(h, cudaStreamSynchronize(ts));
     note_done(h, h->batch_seq);
     h->res_taken[h->batch_seq & 3] = true;
+    return ELLC_OK;
+}
+
+// One batch (sequence number, events, slot read-marks) of `waves` tracking launches on one tracking stream.  The call's own device
+// buffer holds, carved by n: the steps and the wave order (sorted position -> step; staged together in one copy), the pair records
+// the chain kernel writes, the result records and the world poses (indexed by step, i.e. in input order).  The async result ring
+// is not touched.
+int ellc_track_sequence_steps(ellc_handle* h, int32_t n, const ellc_seq_step* steps, ellc_result* results, float* world_poses) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (n < 0 || (n > 0 && (!steps || !results || !world_poses))) { h->err = "bad step list / null outputs"; return ELLC_ERR_INVALID; }
+    if (n == 0) return ELLC_OK;
+    // wave of a step: one after the later of its dependencies (a step whose world poses are both given by value: wave 0)
+    std::vector<int> wave(n);
+    int n_waves = 0;
+    bool save_weights = false, const_weight = false;
+    std::vector<ellc_pair> pairs(n);
+    for (int i = 0; i < n; ++i) {
+        const ellc_seq_step& s = steps[i];
+        if (s.prev_step < -1 || s.prev_step >= i || s.kf_step < -1 || s.kf_step >= i) {
+            h->err = "step " + std::to_string(i) + " depends on a step that does not precede it (-1 <= prev_step, kf_step < i)";
+            return ELLC_ERR_INVALID;
+        }
+        wave[i] = 1 + std::max(s.prev_step < 0 ? -1 : wave[s.prev_step], s.kf_step < 0 ? -1 : wave[s.kf_step]);
+        n_waves = std::max(n_waves, wave[i] + 1);
+        pairs[i].kf_slot = s.kf_slot; pairs[i].frame_slot = s.frame_slot; pairs[i].flags = s.flags;
+        save_weights |= (s.flags & ELLC_PAIR_SAVE_WEIGHTS) != 0;
+        const_weight |= (s.flags & ELLC_PAIR_CONST_WEIGHT) != 0;
+    }
+    int rc = validate_pairs(h, n, pairs.data());
+    if (rc) return rc;
+    // Schedule: by wave, and inside a wave as track_launch orders a batch (forward pairs first, then frame-major, keyframe-minor).
+    // Wave w is [start[2w], start[2w + 2]), its forward pairs [start[2w], start[2w + 1]).
+    auto key = [&](int i) { return 2 * wave[i] + ((steps[i].flags & ELLC_PAIR_CONST_WEIGHT) ? 1 : 0); };
+    std::vector<int> start(2 * n_waves + 1, 0), order(n);
+    for (int i = 0; i < n; ++i) { order[i] = i; ++start[key(i) + 1]; }
+    for (int k = 0; k < 2 * n_waves; ++k) start[k + 1] += start[k];
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) {
+        if (key(a) != key(b)) return key(a) < key(b);
+        if (steps[a].frame_slot != steps[b].frame_slot) return steps[a].frame_slot < steps[b].frame_slot;
+        return steps[a].kf_slot < steps[b].kf_slot;
+    });
+    CU_TRY(h, cudaSetDevice(h->cfg.device));
+    rc = flush_dirty(h);
+    if (rc) return rc;
+    if (save_weights || const_weight) {
+        rc = ensure_lc_pools(h);
+        if (rc) return rc;
+    }
+    long long seq = 0;
+    rc = batch_begin(h, &seq);
+    if (rc) return rc;
+    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t o_order = up((size_t)n * sizeof(ellc_seq_step)), o_pairs = up(o_order + (size_t)n * sizeof(int)),
+                 o_res = up(o_pairs + (size_t)n * sizeof(ellc_pair)), o_world = up(o_res + (size_t)n * sizeof(ellc_result)),
+                 total = o_world + (size_t)n * 6 * sizeof(float);
+    if (total > h->seq_bytes) {                            // (the previous call has completed: it is synchronous)
+        cudaFree(h->d_seq); h->d_seq = nullptr; h->seq_bytes = 0;
+        CU_TRY(h, cudaMalloc(&h->d_seq, total));
+        h->seq_bytes = total;
+    }
+    const ellc_seq_step* d_steps = reinterpret_cast<const ellc_seq_step*>(h->d_seq);
+    const int* d_order = reinterpret_cast<const int*>(h->d_seq + o_order);
+    ellc_pair* d_pairs = reinterpret_cast<ellc_pair*>(h->d_seq + o_pairs);
+    ellc_result* d_res = reinterpret_cast<ellc_result*>(h->d_seq + o_res);
+    float* d_world = reinterpret_cast<float*>(h->d_seq + o_world);
+    rc = batch_order(h, seq, !h->overlap_batches || save_weights || const_weight);
+    if (rc) return rc;
+    cudaStream_t ts = h->tstream[seq & 1];
+    auto enqueue = [&]() -> int {
+        std::vector<char> stage(o_order + (size_t)n * sizeof(int));
+        std::memcpy(stage.data(), steps, (size_t)n * sizeof(ellc_seq_step));
+        std::memcpy(stage.data() + o_order, order.data(), (size_t)n * sizeof(int));
+        int r = stage_h2d_on(h, ts, h->d_seq, stage.data(), stage.size());
+        if (r) return r;
+        CU_TRY(h, cudaEventRecord(h->ev0r[seq & 3], ts));
+        TrackParams p;
+        fill_params(h, p);
+        p.pairs = d_pairs; p.results = d_res;
+        h->launches += launch_seq_init(ts, d_steps, d_order, d_world, d_pairs, 0, start[2]);      // pair records of wave 0
+        for (int w = 0; w < n_waves; ++w) {
+            const int b = start[2 * w], m = start[2 * w + 1], e = start[2 * w + 2];
+            // each wave is scheduled as ellc_track_batch schedules a batch of its pairs: the same cluster / lockstep choice
+            p.order = d_order + b; p.n_pairs = m - b;
+            const int cluster = pick_cluster(h, m - b);
+            p.pairs_per_cta = pick_pairs_per_cta(h, m - b, cluster);
+            int l = launch_track(ts, p, cluster, h->cfg.arithmetic);
+            if (l < 0) { h->err = std::string("track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
+            h->launches += l;
+            if (e > m) {
+                p.order = d_order + m; p.n_pairs = e - m;
+                l = launch_track_lc(ts, p, h->cfg.arithmetic);
+                if (l < 0) { h->err = std::string("loop-closure track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
+                h->launches += l;
+            }
+            h->launches += launch_seq_world(ts, d_steps, d_order, d_res, d_world, b, e);
+            if (w + 1 < n_waves) h->launches += launch_seq_init(ts, d_steps, d_order, d_world, d_pairs, e, start[2 * w + 4]);
+        }
+        CU_TRY(h, cudaGetLastError());
+        return ELLC_OK;
+    };
+    const int enq = enqueue();
+    // The batch is closed and its slots read-marked even when a launch failed part way: the waves already queued still read these
+    // slots, and later uploads / calls must stay ordered behind them.
+    rc = batch_end(h, seq);
+    for (int i = 0; i < n; ++i) { h->fr_reader[steps[i].frame_slot] = seq; h->kf_reader[steps[i].kf_slot] = seq; }
+    if (enq) return enq;
+    if (rc) return rc;
+    CU_TRY(h, cudaMemcpyAsync(results, d_res, (size_t)n * sizeof(ellc_result), cudaMemcpyDeviceToHost, ts));
+    CU_TRY(h, cudaMemcpyAsync(world_poses, d_world, (size_t)n * 6 * sizeof(float), cudaMemcpyDeviceToHost, ts));
+    CU_TRY(h, cudaStreamSynchronize(ts));
+    note_done(h, seq);
     return ELLC_OK;
 }
 

@@ -57,6 +57,13 @@ int launch_invert6(cudaStream_t st, const float* d_in /*H36*/, float* d_out /*Hi
 // one-warp kernel running K5's LU, deltapose / weightedPose and pose update of the given flavour (ellc_solve_update)
 int launch_solve_update(cudaStream_t st, const float* d_in /*H36 b6 pose6 weight6*/, float* d_out /*pose6 delta6 wp1 ok1 rt12 small1*/, int arithmetic);
 
+// ellc_sequence.cu -- pose chain of ellc_track_sequence_steps.  Steps are visited through order[] (sorted position -> step index);
+// [b, e) is one wave: seq_world stores the world poses of a tracked wave, seq_init writes the pair records of the next one.
+int launch_seq_world(cudaStream_t st, const ellc_seq_step* d_steps, const int* d_order, const ellc_result* d_results, float* d_world,
+                     int b, int e);
+int launch_seq_init(cudaStream_t st, const ellc_seq_step* d_steps, const int* d_order, const float* d_world, ellc_pair* d_pairs,
+                    int b, int e);
+
 // ellc_ingest.cu -- camera frame -> level-0 image (gray, undistortion, resize in one pass)
 struct IngestJob { const uint8_t* src; uint8_t* dst; };                 // camera image (device), level-0 image of the slot
 struct IngestGeo { int cam_w, cam_h, channels, pitch, out_w, out_h, undistort, pad; };
