@@ -55,6 +55,18 @@ class SeqStep(C.Structure):
                 ("prev_world", C.c_float * 6), ("kf_world", C.c_float * 6), ("flags", C.c_int32), ("reserved", C.c_int32)]
 
 
+class LcKeyframe(C.Structure):
+    _fields_ = [("kf_slot", C.c_int32), ("frame_slot", C.c_int32), ("frame_id", C.c_int32), ("world_step", C.c_int32),
+                ("world", C.c_float * 6), ("retire_before", C.c_int32), ("ring", C.c_int32), ("ring_pos", C.c_int32),
+                ("current_array_id", C.c_int32), ("match_window_beg", C.c_int32), ("match_window_end", C.c_int32), ("stray", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
+class LcRingParams(C.Structure):
+    _fields_ = [("n_rings", C.c_int32), ("ring_len", C.c_int32), ("min_match_difference", C.c_int32), ("match_threshold", C.c_float),
+                ("max_rel_view_angle", C.c_float), ("reserved", C.c_int32)]
+
+
 class Camera(C.Structure):
     _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("channels", C.c_int32), ("pitch", C.c_int32),
                 ("undistort", C.c_int32), ("reserved", C.c_int32), ("K", C.c_double * 9), ("dist", C.c_double * 5),
@@ -81,6 +93,10 @@ SEQ_STEP_DTYPE = np.dtype([("kf_slot", "<i4"), ("frame_slot", "<i4"), ("prev_ste
                            ("prev_world", "<f4", 6), ("kf_world", "<f4", 6), ("flags", "<i4"), ("reserved", "<i4")])
 assert PAIR_DTYPE.itemsize == 36 and RESULT_DTYPE.itemsize == 256 and TRACE_DTYPE.itemsize == 256
 assert C.sizeof(SeqStep) == SEQ_STEP_DTYPE.itemsize == 72
+LC_KEYFRAME_DTYPE = np.dtype([("kf_slot", "<i4"), ("frame_slot", "<i4"), ("frame_id", "<i4"), ("world_step", "<i4"), ("world", "<f4", 6),
+                              ("retire_before", "<i4"), ("ring", "<i4"), ("ring_pos", "<i4"), ("current_array_id", "<i4"),
+                              ("match_window_beg", "<i4"), ("match_window_end", "<i4"), ("stray", "<i4"), ("reserved", "<i4")])
+assert C.sizeof(LcKeyframe) == LC_KEYFRAME_DTYPE.itemsize == 72 and C.sizeof(LcRingParams) == 24
 
 # every symbol include/ellc_gn.h declares
 SYMBOLS = ["ellc_default_config", "ellc_create", "ellc_destroy", "ellc_last_error_string", "ellc_version",
@@ -97,7 +113,7 @@ SYMBOLS = ["ellc_default_config", "ellc_create", "ellc_destroy", "ellc_last_erro
            "ellc_exchange_wait", "ellc_exchange_destroy", "ellc_se3_exp_closed", "ellc_se3_log_closed",
            "ellc_gn_iterate", "ellc_hessian_inverse", "ellc_lc_generate_pairs", "ellc_track_generated_pairs",
            "ellc_optimal_new_camera_matrix", "ellc_set_camera", "ellc_ingest_frames", "ellc_ingest_keyframe", "ellc_read_camera_tables",
-           "ellc_track_sequence_steps"]
+           "ellc_track_sequence_steps", "ellc_track_sequence_lc"]
 VARIANT_FORWARD, VARIANT_CONST_WEIGHT, VARIANT_PYRAMID = 0, 1, 2
 
 
@@ -193,6 +209,8 @@ def lib():
         L.ellc_read_camera_tables.argtypes = [C.c_void_p] + [C.c_void_p] * 4
         L.ellc_se3_log_closed.argtypes = [C.c_void_p] * 2
         L.ellc_track_sequence_steps.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.ellc_track_sequence_lc.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.POINTER(LcRingParams), C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -444,6 +462,47 @@ class Tracker:
         self._chk(lib().ellc_track_sequence_steps(self._h, n, _p(steps), _p(res), _p(world)))
         self._keep = []
         return res, world
+
+    @staticmethod
+    def make_lc_keyframes(kf_slots, frame_slots, frame_ids, world_steps, world=None, retire_before=-1, ring=0, ring_pos=0,
+                          current_array_id=0, match_window_beg=0, match_window_end=0, stray=0):
+        """An ellc_lc_keyframe array (include/ellc_gn.h); world (n x 6) is only read where world_steps is -1, the ring / query fields
+        only where retire_before >= 0."""
+        n = len(kf_slots)
+        kfs = np.zeros(n, LC_KEYFRAME_DTYPE)
+        for name, v in (("kf_slot", kf_slots), ("frame_slot", frame_slots), ("frame_id", frame_ids), ("world_step", world_steps),
+                        ("retire_before", retire_before), ("ring", ring), ("ring_pos", ring_pos), ("current_array_id", current_array_id),
+                        ("match_window_beg", match_window_beg), ("match_window_end", match_window_end), ("stray", stray)):
+            kfs[name] = v
+        if world is not None:
+            kfs["world"] = np.asarray(world, np.float32).reshape(n, 6)
+        return kfs
+
+    def track_sequence_lc(self, steps, kfs, ring_in, min_match_difference=8, match_threshold=0.1, max_rel_view_angle=10.0):
+        """Sequences in the constant-weight loop-closure mode in one call (ellc_track_sequence_lc).  ring_in: (n_rings, ring_len)
+        LC_RING_DTYPE array, the rings before the call.  Returns a dict of numpy arrays: results and world (the steps, input order),
+        lc_pairs, lc_stats, lc_query_of_pair (index into kfs), lc_results (the loop-closure pairs, query-major in push order) and
+        ring_out (the rings after the call, the ring_in of the next call)."""
+        steps = np.ascontiguousarray(steps, SEQ_STEP_DTYPE)
+        kfs = np.ascontiguousarray(kfs, LC_KEYFRAME_DTYPE)
+        ring_in = np.ascontiguousarray(ring_in, LC_RING_DTYPE)
+        if ring_in.ndim != 2:
+            raise EllcError("ring_in must be (n_rings, ring_len)")
+        n_rings, ring_len = ring_in.shape
+        n, cap = len(steps), max(1, int((kfs["retire_before"] >= 0).sum()) * ring_len)
+        res = np.zeros(n, RESULT_DTYPE)
+        world = np.zeros((n, 6), np.float32)
+        pairs = np.zeros(cap, PAIR_DTYPE); stats = np.zeros(cap, LC_STATS_DTYPE); qi = np.zeros(cap, np.int32)
+        lres = np.zeros(cap, RESULT_DTYPE)
+        ring_out = np.zeros_like(ring_in)
+        rp = LcRingParams(n_rings, ring_len, int(min_match_difference), float(match_threshold), float(max_rel_view_angle), 0)
+        m = C.c_int32()
+        self._chk(lib().ellc_track_sequence_lc(self._h, n, _p(steps), len(kfs), _p(kfs), C.byref(rp), _p(ring_in), _p(res), _p(world),
+                                               C.byref(m), _p(pairs), _p(stats), _p(qi), _p(lres), _p(ring_out)))
+        self._keep = []
+        k = m.value
+        return dict(results=res, world=world, lc_pairs=pairs[:k], lc_stats=stats[:k], lc_query_of_pair=qi[:k], lc_results=lres[:k],
+                    ring_out=ring_out)
 
     def track_batch_async(self, pairs):
         pairs = np.ascontiguousarray(pairs, PAIR_DTYPE)

@@ -1282,14 +1282,28 @@ int ellc_track_batch(ellc_handle* h, int32_t n, const ellc_pair* pairs, ellc_res
     return ELLC_OK;
 }
 
+}  // extern "C"
+
+// The loop-closure part of ellc_track_sequence_lc, validated by its caller; null for ellc_track_sequence_steps.
+struct SeqLc {
+    int n_kf;
+    const ellc_lc_keyframe* kfs;
+    ellc_lc_ring_params rp;
+    const ellc_lc_ring_entry* ring_in;
+    int32_t* n_pairs; ellc_pair* pairs; ellc_lc_stats* stats; int32_t* query_of_pair; ellc_result* lc_results;
+    ellc_lc_ring_entry* ring_out;
+    std::vector<int> list_off;                             // start of every keyframe's frame list; last entry: total length
+    std::vector<int> n_frames;                             // its length (ELLC_PAIR_SAVE_WEIGHTS steps naming the keyframe)
+    std::vector<int> ret_kf, ret_fr;                       // kf / frame slots of the retired keyframes, in push order
+};
+
 // One batch (sequence number, events, slot read-marks) of `waves` tracking launches on one tracking stream.  The call's own device
 // buffer holds, carved by n: the steps and the wave order (sorted position -> step; staged together in one copy), the pair records
 // the chain kernel writes, the result records and the world poses (indexed by step, i.e. in input order).  The async result ring
-// is not touched.
-int ellc_track_sequence_steps(ellc_handle* h, int32_t n, const ellc_seq_step* steps, ellc_result* results, float* world_poses) {
-    if (!h) return ELLC_ERR_INVALID;
-    if (n < 0 || (n > 0 && (!steps || !results || !world_poses))) { h->err = "bad step list / null outputs"; return ELLC_ERR_INVALID; }
-    if (n == 0) return ELLC_OK;
+// is not touched.  With lc, the loop-closure inputs are staged in the same copy and the keyframe / ring phase runs on the same
+// stream after the last wave: frame lists, weights, loop-closure records, histograms, pushes, walk and pack; then one wait for the
+// number of pairs, and their tracking.
+static int track_sequence_impl(ellc_handle* h, int32_t n, const ellc_seq_step* steps, ellc_result* results, float* world_poses, SeqLc* lc) {
     // wave of a step: one after the later of its dependencies (a step whose world poses are both given by value: wave 0)
     std::vector<int> wave(n);
     int n_waves = 0;
@@ -1320,44 +1334,75 @@ int ellc_track_sequence_steps(ellc_handle* h, int32_t n, const ellc_seq_step* st
         if (steps[a].frame_slot != steps[b].frame_slot) return steps[a].frame_slot < steps[b].frame_slot;
         return steps[a].kf_slot < steps[b].kf_slot;
     });
+    const int n_kf = lc ? lc->n_kf : 0, n_ret = lc ? (int)lc->ret_kf.size() : 0;
+    const int ring_len = lc ? lc->rp.ring_len : 0, n_ring_e = lc ? lc->rp.n_rings * lc->rp.ring_len : 0;
     CU_TRY(h, cudaSetDevice(h->cfg.device));
     rc = flush_dirty(h);
     if (rc) return rc;
-    if (save_weights || const_weight) {
+    if (save_weights || const_weight || n_kf > 0) {
         rc = ensure_lc_pools(h);
         if (rc) return rc;
     }
+    if (n_ret > 0 && !h->fr_hist) CU_TRY(h, cudaMalloc(&h->fr_hist, (size_t)h->cfg.max_frames * 256 * sizeof(float)));
     long long seq = 0;
     rc = batch_begin(h, &seq);
     if (rc) return rc;
     auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t o_order = up((size_t)n * sizeof(ellc_seq_step)), o_pairs = up(o_order + (size_t)n * sizeof(int)),
+    // loop-closure inputs, staged behind the order: keyframes, ring_in, prior counts [k][level], list offsets, retired kf / frame slots
+    const size_t l_kfs = 0, l_ring = up(l_kfs + (size_t)n_kf * sizeof(ellc_lc_keyframe)), l_prior = up(l_ring + (size_t)n_ring_e * sizeof(ellc_lc_ring_entry)),
+                 l_off = up(l_prior + (size_t)n_kf * kLevels * sizeof(int)), l_rkf = up(l_off + (size_t)n_kf * sizeof(int)),
+                 l_rfr = up(l_rkf + (size_t)n_ret * sizeof(int)), lc_in = lc ? l_rfr + (size_t)n_ret * sizeof(int) : 0;
+    const size_t o_order = up((size_t)n * sizeof(ellc_seq_step)), o_lcin = up(o_order + (size_t)n * sizeof(int)), o_pairs = up(o_lcin + lc_in),
                  o_res = up(o_pairs + (size_t)n * sizeof(ellc_pair)), o_world = up(o_res + (size_t)n * sizeof(ellc_result)),
-                 total = o_world + (size_t)n * 6 * sizeof(float);
+                 seq_end = o_world + (size_t)n * 6 * sizeof(float);
+    // loop-closure outputs and scratch: frame lists, their lengths, pushes, queries, per-query segments, the packed list, its records,
+    // the rings after the call
+    const size_t cap = (size_t)n_kf * ring_len, n_lists = lc ? (size_t)lc->list_off[n_kf] : 0;
+    const size_t o_lists = up(seq_end), o_cnt = up(o_lists + n_lists * sizeof(int)), o_push = up(o_cnt + (size_t)n_kf * sizeof(int)),
+                 o_q = up(o_push + (size_t)n_kf * sizeof(ellc_lc_ring_entry)), o_segp = up(o_q + (size_t)n_kf * sizeof(ellc_lc_query)),
+                 o_segs = up(o_segp + cap * sizeof(ellc_pair)), o_segc = up(o_segs + cap * sizeof(ellc_lc_stats)),
+                 o_lp = up(o_segc + (size_t)n_kf * sizeof(int)), o_ls = up(o_lp + cap * sizeof(ellc_pair)), o_lq = up(o_ls + cap * sizeof(ellc_lc_stats)),
+                 o_tot = up(o_lq + cap * sizeof(int)), o_lres = up(o_tot + sizeof(int)), o_rout = up(o_lres + cap * sizeof(ellc_result)),
+                 total = lc ? o_rout + (size_t)n_ring_e * sizeof(ellc_lc_ring_entry) : seq_end;
     if (total > h->seq_bytes) {                            // (the previous call has completed: it is synchronous)
         cudaFree(h->d_seq); h->d_seq = nullptr; h->seq_bytes = 0;
         CU_TRY(h, cudaMalloc(&h->d_seq, total));
         h->seq_bytes = total;
     }
-    const ellc_seq_step* d_steps = reinterpret_cast<const ellc_seq_step*>(h->d_seq);
-    const int* d_order = reinterpret_cast<const int*>(h->d_seq + o_order);
-    ellc_pair* d_pairs = reinterpret_cast<ellc_pair*>(h->d_seq + o_pairs);
-    ellc_result* d_res = reinterpret_cast<ellc_result*>(h->d_seq + o_res);
-    float* d_world = reinterpret_cast<float*>(h->d_seq + o_world);
-    rc = batch_order(h, seq, !h->overlap_batches || save_weights || const_weight);
+    char* const d = h->d_seq;
+    const ellc_seq_step* d_steps = reinterpret_cast<const ellc_seq_step*>(d);
+    const int* d_order = reinterpret_cast<const int*>(d + o_order);
+    ellc_pair* d_pairs = reinterpret_cast<ellc_pair*>(d + o_pairs);
+    ellc_result* d_res = reinterpret_cast<ellc_result*>(d + o_res);
+    float* d_world = reinterpret_cast<float*>(d + o_world);
+    rc = batch_order(h, seq, !h->overlap_batches || save_weights || const_weight || lc != nullptr);
     if (rc) return rc;
     cudaStream_t ts = h->tstream[seq & 1];
+    int n_lc = 0;
     auto enqueue = [&]() -> int {
-        std::vector<char> stage(o_order + (size_t)n * sizeof(int));
+        std::vector<char> stage(o_lcin + lc_in);
         std::memcpy(stage.data(), steps, (size_t)n * sizeof(ellc_seq_step));
         std::memcpy(stage.data() + o_order, order.data(), (size_t)n * sizeof(int));
+        if (lc) {
+            char* L = stage.data() + o_lcin;
+            std::memcpy(L + l_kfs, lc->kfs, (size_t)n_kf * sizeof(ellc_lc_keyframe));
+            if (n_ring_e) std::memcpy(L + l_ring, lc->ring_in, (size_t)n_ring_e * sizeof(ellc_lc_ring_entry));
+            int* prior = reinterpret_cast<int*>(L + l_prior);
+            for (int k = 0; k < n_kf; ++k)
+                for (int l = 0; l < kLevels; ++l) prior[kLevels * k + l] = h->kf_wcount[(size_t)lc->kfs[k].kf_slot * kLevels + l];
+            std::memcpy(L + l_off, lc->list_off.data(), (size_t)n_kf * sizeof(int));
+            if (n_ret) {
+                std::memcpy(L + l_rkf, lc->ret_kf.data(), (size_t)n_ret * sizeof(int));
+                std::memcpy(L + l_rfr, lc->ret_fr.data(), (size_t)n_ret * sizeof(int));
+            }
+        }
         int r = stage_h2d_on(h, ts, h->d_seq, stage.data(), stage.size());
         if (r) return r;
         CU_TRY(h, cudaEventRecord(h->ev0r[seq & 3], ts));
         TrackParams p;
         fill_params(h, p);
         p.pairs = d_pairs; p.results = d_res;
-        h->launches += launch_seq_init(ts, d_steps, d_order, d_world, d_pairs, 0, start[2]);      // pair records of wave 0
+        if (n_waves > 0) h->launches += launch_seq_init(ts, d_steps, d_order, d_world, d_pairs, 0, start[2]);      // pair records of wave 0
         for (int w = 0; w < n_waves; ++w) {
             const int b = start[2 * w], m = start[2 * w + 1], e = start[2 * w + 2];
             // each wave is scheduled as ellc_track_batch schedules a batch of its pairs: the same cluster / lockstep choice
@@ -1377,6 +1422,50 @@ int ellc_track_sequence_steps(ellc_handle* h, int32_t n, const ellc_seq_step* st
             if (w + 1 < n_waves) h->launches += launch_seq_init(ts, d_steps, d_order, d_world, d_pairs, e, start[2 * w + 4]);
         }
         CU_TRY(h, cudaGetLastError());
+        if (!lc) return ELLC_OK;
+        // ---- keyframes: weights (all listed), then loop-closure records and histograms of the retired ones
+        const char* L = d + o_lcin;
+        const ellc_lc_keyframe* d_kfs = reinterpret_cast<const ellc_lc_keyframe*>(L + l_kfs);
+        const ellc_lc_ring_entry* d_ring_in = reinterpret_cast<const ellc_lc_ring_entry*>(L + l_ring);
+        const int* d_off = reinterpret_cast<const int*>(L + l_off);
+        int* d_lists = reinterpret_cast<int*>(d + o_lists);
+        int* d_cnt = reinterpret_cast<int*>(d + o_cnt);
+        h->launches += launch_seq_kf_lists(ts, d_steps, n, d_kfs, n_kf, d_off, d_lists, d_cnt);
+        h->launches += launch_seq_kf_weights(ts, h->kf_weight, h->kf_mask, h->fr_weight, d_kfs, n_kf, d_off, d_lists, d_cnt,
+                                             reinterpret_cast<const int*>(L + l_prior), h->geo);
+        CU_TRY(h, cudaGetLastError());
+        if (n_ret == 0) return ELLC_OK;
+        const int* d_rkf = reinterpret_cast<const int*>(L + l_rkf);
+        h->launches += launch_lc_prepare(ts, h->kf_geo, h->kf_pix, h->geo.win_off[kLevels], h->kf_count, h->kf_img, h->geo.img_off[kLevels],
+                                         h->kf_weight, h->kf_lc, h->kf_lcf, h->kf_lcp, h->kf_lcH, h->K, d_rkf, n_ret, h->geo,
+                                         h->cfg.arithmetic == ELLC_ARITH_REFERENCE);
+        h->launches += launch_frame_histograms(ts, h->fr_img, h->geo.img_off[kLevels], reinterpret_cast<const int*>(L + l_rfr), n_ret,
+                                               h->geo.width * h->geo.height, h->fr_hist);
+        // ---- ring: pushes with the chain's world poses, the walk of every query on its ring as of its push, the packed pair list
+        ellc_lc_ring_entry* d_push = reinterpret_cast<ellc_lc_ring_entry*>(d + o_push);
+        ellc_lc_query* d_q = reinterpret_cast<ellc_lc_query*>(d + o_q);
+        h->launches += launch_seq_ring_push(ts, d_kfs, n_kf, d_world, d_ring_in, lc->rp.n_rings, ring_len, d_push, d_q,
+                                            reinterpret_cast<ellc_lc_ring_entry*>(d + o_rout));
+        const int l = launch_lc_generate_seq(ts, h->fr_hist, d_ring_in, ring_len, d_kfs, n_kf, d_push, d_q, lc->rp.min_match_difference,
+                                             lc->rp.match_threshold, lc->rp.max_rel_view_angle, ELLC_PAIR_CONST_WEIGHT,
+                                             reinterpret_cast<ellc_pair*>(d + o_segp), reinterpret_cast<ellc_lc_stats*>(d + o_segs),
+                                             reinterpret_cast<int*>(d + o_segc), reinterpret_cast<ellc_pair*>(d + o_lp),
+                                             reinterpret_cast<ellc_lc_stats*>(d + o_ls), reinterpret_cast<int*>(d + o_lq), reinterpret_cast<int*>(d + o_tot));
+        if (l < 0) { h->err = "pair-list kernels: bad launch configuration"; return ELLC_ERR_INVALID; }
+        h->launches += l;
+        CU_TRY(h, cudaGetLastError());
+        // ---- the loop-closure pairs: the one wait of the call, for their number (the grid size), then their tracking
+        CU_TRY(h, cudaMemcpyAsync(&n_lc, d + o_tot, sizeof(int), cudaMemcpyDeviceToHost, ts));
+        CU_TRY(h, cudaStreamSynchronize(ts));
+        if (n_lc > 0) {
+            TrackParams q;
+            fill_params(h, q);
+            q.pairs = reinterpret_cast<const ellc_pair*>(d + o_lp); q.order = nullptr; q.results = reinterpret_cast<ellc_result*>(d + o_lres);
+            q.n_pairs = n_lc;
+            const int lt = launch_track_lc(ts, q, h->cfg.arithmetic);
+            if (lt < 0) { h->err = std::string("loop-closure track kernel launch failed: ") + cudaGetErrorString(cudaGetLastError()); return ELLC_ERR_CUDA; }
+            h->launches += lt;
+        }
         return ELLC_OK;
     };
     const int enq = enqueue();
@@ -1384,13 +1473,125 @@ int ellc_track_sequence_steps(ellc_handle* h, int32_t n, const ellc_seq_step* st
     // slots, and later uploads / calls must stay ordered behind them.
     rc = batch_end(h, seq);
     for (int i = 0; i < n; ++i) { h->fr_reader[steps[i].frame_slot] = seq; h->kf_reader[steps[i].kf_slot] = seq; }
+    if (lc) {
+        for (int k = 0; k < n_kf; ++k) { h->fr_reader[lc->kfs[k].frame_slot] = seq; h->kf_reader[lc->kfs[k].kf_slot] = seq; }
+        for (int i = 0; i < n_ring_e; ++i)
+            if (lc->ring_in[i].is_valid) { h->fr_reader[lc->ring_in[i].frame_slot] = seq; h->kf_reader[lc->ring_in[i].kf_slot] = seq; }
+        // the weights were written (as ellc_accumulate_weights / _finalise_weights / ellc_prepare_keyframes_lc leave them)
+        for (int k = 0; k < n_kf; ++k) {
+            const int ks = lc->kfs[k].kf_slot;
+            for (int l = 0; l < kLevels; ++l) h->kf_wcount[(size_t)ks * kLevels + l] += lc->n_frames[k];
+            if (lc->n_frames[k] > 0 || lc->kfs[k].retire_before >= 0) h->kf_lc_ready[ks] = 0;
+        }
+        if (!enq) {
+            for (int ks : lc->ret_kf) h->kf_lc_ready[ks] = 1;
+            for (int fs : lc->ret_fr) h->fr_hist_ready[fs] = 1;
+        }
+    }
     if (enq) return enq;
     if (rc) return rc;
     CU_TRY(h, cudaMemcpyAsync(results, d_res, (size_t)n * sizeof(ellc_result), cudaMemcpyDeviceToHost, ts));
     CU_TRY(h, cudaMemcpyAsync(world_poses, d_world, (size_t)n * 6 * sizeof(float), cudaMemcpyDeviceToHost, ts));
+    if (lc) {
+        *lc->n_pairs = n_lc;
+        if (n_lc > 0) {
+            if (lc->pairs) CU_TRY(h, cudaMemcpyAsync(lc->pairs, d + o_lp, (size_t)n_lc * sizeof(ellc_pair), cudaMemcpyDeviceToHost, ts));
+            if (lc->stats) CU_TRY(h, cudaMemcpyAsync(lc->stats, d + o_ls, (size_t)n_lc * sizeof(ellc_lc_stats), cudaMemcpyDeviceToHost, ts));
+            if (lc->query_of_pair) CU_TRY(h, cudaMemcpyAsync(lc->query_of_pair, d + o_lq, (size_t)n_lc * sizeof(int), cudaMemcpyDeviceToHost, ts));
+            if (lc->lc_results) CU_TRY(h, cudaMemcpyAsync(lc->lc_results, d + o_lres, (size_t)n_lc * sizeof(ellc_result), cudaMemcpyDeviceToHost, ts));
+        }
+        if (n_ring_e) {
+            if (n_ret > 0) CU_TRY(h, cudaMemcpyAsync(lc->ring_out, d + o_rout, (size_t)n_ring_e * sizeof(ellc_lc_ring_entry), cudaMemcpyDeviceToHost, ts));
+            else std::memmove(lc->ring_out, lc->ring_in, (size_t)n_ring_e * sizeof(ellc_lc_ring_entry));
+        }
+    }
     CU_TRY(h, cudaStreamSynchronize(ts));
     note_done(h, seq);
     return ELLC_OK;
+}
+
+extern "C" {
+
+int ellc_track_sequence_steps(ellc_handle* h, int32_t n, const ellc_seq_step* steps, ellc_result* results, float* world_poses) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (n < 0 || (n > 0 && (!steps || !results || !world_poses))) { h->err = "bad step list / null outputs"; return ELLC_ERR_INVALID; }
+    if (n == 0) return ELLC_OK;
+    return track_sequence_impl(h, n, steps, results, world_poses, nullptr);
+}
+
+int ellc_track_sequence_lc(ellc_handle* h, int32_t n, const ellc_seq_step* steps, int32_t n_kf, const ellc_lc_keyframe* kfs,
+                           const ellc_lc_ring_params* ring_params, const ellc_lc_ring_entry* ring_in,
+                           ellc_result* results, float* world_poses, int32_t* n_lc_pairs, ellc_pair* lc_pairs, ellc_lc_stats* lc_stats,
+                           int32_t* lc_query_of_pair, ellc_result* lc_results, ellc_lc_ring_entry* ring_out) {
+    if (!h) return ELLC_ERR_INVALID;
+    if (n < 0 || n_kf < 0 || (n > 0 && (!steps || !results || !world_poses)) || (n_kf > 0 && !kfs) || !ring_params || !n_lc_pairs) {
+        h->err = "bad step / keyframe lists or null outputs";
+        return ELLC_ERR_INVALID;
+    }
+    *n_lc_pairs = 0;
+    const ellc_lc_ring_params& rp = *ring_params;
+    if (rp.n_rings < 0 || (rp.n_rings > 0 && (rp.ring_len < 1 || rp.ring_len > 64 || !ring_in || !ring_out))) {
+        h->err = "bad ring parameters (1 <= ring_len <= 64, ring_in / ring_out of n_rings x ring_len entries)";
+        return ELLC_ERR_INVALID;
+    }
+    SeqLc lc;
+    lc.n_kf = n_kf; lc.kfs = kfs; lc.rp = rp; lc.ring_in = ring_in;
+    lc.n_pairs = n_lc_pairs; lc.pairs = lc_pairs; lc.stats = lc_stats; lc.query_of_pair = lc_query_of_pair; lc.lc_results = lc_results;
+    lc.ring_out = ring_out;
+    if (rp.n_rings == 0) lc.rp.ring_len = 0;
+    // keyframes: slots, world dependency, retirement, ring fields
+    std::vector<int> kf_index(h->cfg.max_keyframes, -1);
+    for (int k = 0; k < n_kf; ++k) {
+        const ellc_lc_keyframe& kf = kfs[k];
+        const std::string at = "keyframe entry " + std::to_string(k) + ": ";
+        if (kf.kf_slot < 0 || kf.kf_slot >= h->cfg.max_keyframes || kf.frame_slot < 0 || kf.frame_slot >= h->cfg.max_frames) {
+            h->err = at + "slot out of range"; return ELLC_ERR_INVALID;
+        }
+        if (kf_index[kf.kf_slot] >= 0) { h->err = at + "keyframe slot listed twice"; return ELLC_ERR_INVALID; }
+        kf_index[kf.kf_slot] = k;
+        if (h->kf_state[kf.kf_slot] == 0 || h->fr_state[kf.frame_slot] == 0) { h->err = at + "slot never uploaded"; return ELLC_ERR_NOT_READY; }
+        if (kf.world_step < -1 || kf.world_step >= n) { h->err = at + "world_step out of range (-1 <= world_step < n)"; return ELLC_ERR_INVALID; }
+        if (kf.retire_before < -1 || kf.retire_before > n) { h->err = at + "retire_before out of range (-1 .. n)"; return ELLC_ERR_INVALID; }
+        if (kf.retire_before < 0) continue;
+        const int L = rp.ring_len;
+        if (kf.ring < 0 || kf.ring >= rp.n_rings || kf.ring_pos < 0 || kf.ring_pos >= L || kf.current_array_id < 0 || kf.current_array_id > L ||
+            kf.match_window_beg < 0 || kf.match_window_beg >= L || kf.match_window_end < 0 || kf.match_window_end >= L) {
+            h->err = at + "ring / ring position / query window out of range"; return ELLC_ERR_INVALID;
+        }
+        lc.ret_kf.push_back(kf.kf_slot); lc.ret_fr.push_back(kf.frame_slot);
+    }
+    // steps: no step may track against a keyframe after its retirement; frame-list lengths
+    lc.n_frames.assign(n_kf, 0);
+    for (int i = 0; i < n; ++i) {
+        const int ks = steps[i].kf_slot;
+        if (ks < 0 || ks >= h->cfg.max_keyframes || kf_index[ks] < 0) continue;      // (slots are checked with the steps)
+        const ellc_lc_keyframe& kf = kfs[kf_index[ks]];
+        if (kf.retire_before >= 0 && i >= kf.retire_before) {
+            h->err = "step " + std::to_string(i) + " tracks against keyframe entry " + std::to_string(kf_index[ks]) + ", which is retired before it";
+            return ELLC_ERR_INVALID;
+        }
+        if (steps[i].flags & ELLC_PAIR_SAVE_WEIGHTS) ++lc.n_frames[kf_index[ks]];
+    }
+    lc.list_off.assign(n_kf + 1, 0);
+    for (int k = 0; k < n_kf; ++k) lc.list_off[k + 1] = lc.list_off[k] + lc.n_frames[k];
+    // the rings before the call: what ellc_lc_generate_pairs requires of a ring
+    for (int i = 0; i < rp.n_rings * lc.rp.ring_len; ++i) {
+        if (!ring_in[i].is_valid) continue;
+        const int fs = ring_in[i].frame_slot, ks = ring_in[i].kf_slot;
+        if (fs < 0 || fs >= h->cfg.max_frames || ks < 0 || ks >= h->cfg.max_keyframes) { h->err = "ring entry references a slot out of range"; return ELLC_ERR_INVALID; }
+        if (!h->fr_hist || !h->fr_hist_ready[fs]) { h->err = "ring entry without histogram: call ellc_frame_histograms first"; return ELLC_ERR_NOT_READY; }
+        if (h->kf_state[ks] == 0) { h->err = "ring entry references a keyframe slot that was never uploaded"; return ELLC_ERR_NOT_READY; }
+        const bool retired_here = kf_index[ks] >= 0 && kfs[kf_index[ks]].retire_before >= 0;
+        if (!h->kf_lc_ready[ks] && !retired_here) {
+            h->err = "ring entry on a keyframe without finalised weights and loop-closure records (ellc_prepare_keyframes_lc)";
+            return ELLC_ERR_NOT_READY;
+        }
+    }
+    if (n == 0 && n_kf == 0) {
+        if (rp.n_rings > 0) std::memmove(ring_out, ring_in, (size_t)rp.n_rings * rp.ring_len * sizeof(ellc_lc_ring_entry));
+        return ELLC_OK;
+    }
+    return track_sequence_impl(h, n, steps, results, world_poses, &lc);
 }
 
 int ellc_gn_iterate(ellc_handle* h, int32_t kf_slot, int32_t frame_slot, int32_t level, int32_t variant, int32_t update,

@@ -23,6 +23,11 @@ int launch_lc_generate(cudaStream_t st, const float* hist_pool, const ellc_lc_ri
                        int n_queries, int min_match_difference, float match_threshold, float max_rel_view_angle, int pair_flags,
                        ellc_pair* d_seg_pairs, ellc_lc_stats* d_seg_stats, int* d_seg_count, ellc_pair* d_pairs, ellc_lc_stats* d_stats,
                        int* d_query_of_pair, int* d_total);
+// ellc_track_sequence_lc: the same walk and packing, every listed keyframe k a query on its ring as of its own push (queries = n_kf)
+int launch_lc_generate_seq(cudaStream_t st, const float* hist_pool, const ellc_lc_ring_entry* d_ring_in, int ring_len, const ellc_lc_keyframe* d_kfs,
+                           int n_kf, const ellc_lc_ring_entry* d_push, const ellc_lc_query* d_queries, int min_match_difference,
+                           float match_threshold, float max_rel_view_angle, int pair_flags, ellc_pair* d_seg_pairs, ellc_lc_stats* d_seg_stats,
+                           int* d_seg_count, ellc_pair* d_pairs, ellc_lc_stats* d_stats, int* d_query_of_pair, int* d_total);
 int launch_lc_gate(cudaStream_t st, const float* hist_pool, const ellc_lc_candidate* d_cand, int n, float match_threshold,
                    float max_rel_view_angle, ellc_lc_stats* d_out);
 // keyframe depth / variance pyramids from hypotheses (src/DepthPropagation.cpp:1254-1306, :1637-1719); depth_slot / var_slot are
@@ -63,6 +68,15 @@ int launch_seq_world(cudaStream_t st, const ellc_seq_step* d_steps, const int* d
                      int b, int e);
 int launch_seq_init(cudaStream_t st, const ellc_seq_step* d_steps, const int* d_order, const float* d_world, ellc_pair* d_pairs,
                     int b, int e);
+// ellc_track_sequence_lc (include/ellc_gn.h): per listed keyframe the frame list of its ELLC_PAIR_SAVE_WEIGHTS steps in step order
+// (at d_list_off[k], count d_count[k]), accumulation + finalisation of its weight pyramid (finalised when retired; d_prior: its
+// counts before the call, [k][level]), and the ring pushes: entries / queries of the retired keyframes, the rings after the call
+int launch_seq_kf_lists(cudaStream_t st, const ellc_seq_step* d_steps, int n, const ellc_lc_keyframe* d_kfs, int n_kf, const int* d_list_off,
+                        int* d_lists, int* d_count);
+int launch_seq_kf_weights(cudaStream_t st, float* kf_weight, const uint8_t* kf_mask, const float* frw_pool, const ellc_lc_keyframe* d_kfs, int n_kf,
+                          const int* d_list_off, const int* d_lists, const int* d_count, const int* d_prior, const Geometry& geo);
+int launch_seq_ring_push(cudaStream_t st, const ellc_lc_keyframe* d_kfs, int n_kf, const float* d_world, const ellc_lc_ring_entry* d_ring_in,
+                         int n_rings, int ring_len, ellc_lc_ring_entry* d_push, ellc_lc_query* d_queries, ellc_lc_ring_entry* d_ring_out);
 
 // ellc_ingest.cu -- camera frame -> level-0 image (gray, undistortion, resize in one pass)
 struct IngestJob { const uint8_t* src; uint8_t* dst; };                 // camera image (device), level-0 image of the slot
